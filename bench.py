@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- frames/s of the per-frame pixel hot path on N B200s, with roofline and CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], "C2"): ZED 2208x1242 stereo frames through balance() (default
@@ -116,6 +116,16 @@ def make_ring(n, h=H, w=W, seed0=2000):
     return np.stack([synth.gen_underwater(h, w, seed0 + i) for i in range(n)])
 
 
+# image rows that --dump-outputs writes of every frame: a fixed, seeded sample (64 frames x 16 rows of LAB = 27 MB float32)
+DUMP_ROWS = np.sort(np.random.default_rng(0).permutation(H)[:16])
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 # ------------------------------------------------------------------------------------------------
 # reference arm: the reference's own CPU implementation on the host cores
 # ------------------------------------------------------------------------------------------------
@@ -176,10 +186,12 @@ def run_reference(args):
         for s in range(args.warmup + args.steps):
             frames = ring[(s % 2) * per_step:(s % 2 + 1) * per_step]
             t0 = time.perf_counter()
-            cpu_reference_step(frames, pool)
+            converted = cpu_reference_step(frames, pool)
             dt = time.perf_counter() - t0
             if s >= args.warmup:
                 times.append(dt)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"converted": np.stack(converted[:BATCH])[:, DUMP_ROWS]})
     total = sum(times)
     value = per_step * args.steps / total
     line = {
@@ -456,6 +468,7 @@ def run_ours(args):
     # synthetic ring, distinct per rank (frame f of the global stream goes to rank f mod world)
     ring_np = make_ring(RING // 2, seed0=2000 + 100 * rank)
     ring = torch.cat([ctx.upload(ring_np), ctx.upload(np.roll(ring_np, 211, axis=2))])
+    dump_rows = torch.from_numpy(DUMP_ROWS).to(ring.device) if (args.dump_outputs and rank == 0) else None
     n_batches = RING // BATCH
     desc = ctx.make_stage(balance={}, cvt="bgr2lab")
     out = {}
@@ -497,6 +510,11 @@ def run_ours(args):
     launches0 = ctx.launches
     elapsed = timed_steps(args.steps, args.warmup)
     launches = ctx.launches - launches0
+    if dump_rows is not None:
+        # the LAB images the last timed step returned: a device copy of the sampled rows, taken before the sustained
+        # repetition below overwrites `out` and written to disk once the clock-sampled window is over
+        with torch.cuda.stream(ctx.torch_stream):
+            dumped = out["converted"].index_select(1, dump_rows)
     value = world * BATCH * args.steps / elapsed
     # the same step repeated for >= ~1.5 s: what a continuously running consumer sees (clocks, power cap)
     sus_steps = int(min(20000, max(args.steps, args.sustain_s / (elapsed / args.steps))))
@@ -504,6 +522,9 @@ def run_ours(args):
     sustained = {"value": world * BATCH * sus_steps / sus_elapsed, "unit": "frames/s", "steps": sus_steps,
                  "seconds": sus_elapsed}
     mark_b = sampler.mark()
+    if dump_rows is not None:
+        write_outputs(args.dump_outputs, {"converted": ctx.download(dumped)})
+        del dumped
 
     # ---- per-kernel timing (library profiler: CUDA events around every launch) ----
     ctx.profile(True)
@@ -723,7 +744,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg (tuning sweeps only)")
     ap.add_argument("--sustain-s", dest="sustain_s", type=float, default=1.5,
                     help="seconds of back-to-back steps for the `sustained` value")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32, a fixed sample of 16 image "
+                         "rows of every frame, at most 27 MB; rank 0 only).  --impl reference: the first 64 frames of "
+                         "its last step, which holds one frame per host core, so its frames follow the host")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -5,7 +5,15 @@
                     /root/reference/utils/color_correction/color_balance.cpp compiled by
                     oracle/Makefile and called exactly like modules/color_balance.py:93-110;
   * cv_*.npz        input + outputs of the literal cv2 calls the reference makes (oracle/cv_ops.py)
-                    with the installed cv2 (third-party dependency of the reference).
+                    with the installed cv2 (third-party dependency of the reference);
+  * process_frame_outputs.npz
+                    process_frame on the frames of the compiled-reference tests in tests/test_oracle_ref.py
+                    (larger frames, HSI branch), too large to store whole: per frame the SHA-256 of input and
+                    output, four full output rows and the source of the output.  `python tests/golden/make_golden.py
+                    process_frame_outputs` takes them from the compiled reference; with --from-restatement (no
+                    reference checkout at hand) from oracle/color_balance_np.py, which those tests compare with the
+                    compiled reference byte for byte.  The stored file says which; test_compiled_reference_reproduces_golden
+                    re-checks it against the compiled reference wherever that is built.
 
 The reference repository has no tests or fixtures of its own (build.ninja:72-73), so these
 vectors are what pins the oracle; they travel to the GPU box, /root/reference does not.
@@ -42,7 +50,32 @@ def load_reference_color():
     return mod
 
 
+def write_process_frame_outputs(from_restatement):
+    sys.path.insert(0, os.path.dirname(OUT))
+    from oracle import color_balance_np
+    from test_oracle_ref import STORED_OUTPUTS, sha256, stored_cases, synth_frame
+    if from_restatement:
+        balance = color_balance_np.process_frame_np
+        source = ("oracle/color_balance_np.py (equal byte for byte to the compiled color_balance.cpp on this input in "
+                  "test_restatement_matches_compiled_reference / test_hsi_branch_restatement_matches_compiled_reference)")
+    else:
+        assert ref_balance.available(), "build oracle/_ref first (make -C oracle), or pass --from-restatement"
+        balance, source = ref_balance.balance, "compiled color_balance.cpp (oracle/_ref)"
+    d = {}
+    for key, (kind, shape, seed, flags) in stored_cases().items():
+        img = synth_frame(kind, shape, seed)
+        out = balance(img, **flags)
+        rows = np.linspace(0, shape[0] - 1, 4).round().astype(np.int64)
+        d.update({key + "__src_sha256": np.array(sha256(img)), key + "__out_sha256": np.array(sha256(out)),
+                  key + "__row_index": rows, key + "__rows": out[rows], key + "__source": np.array(source)})
+    np.savez_compressed(STORED_OUTPUTS, **d)
+    print("wrote", STORED_OUTPUTS, "from", source)
+
+
 def main():
+    if len(sys.argv) > 1 and sys.argv[1] == "process_frame_outputs":
+        write_process_frame_outputs("--from-restatement" in sys.argv)
+        return
     assert ref_balance.available(), "build oracle/_ref first (make -C oracle)"
     # colour balance: default flags on three shapes (one with width % 32 != 0), plus flag variants
     cases = [("default_96x160", 96, 160, 11, {}),
