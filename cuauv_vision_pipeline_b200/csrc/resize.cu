@@ -382,6 +382,8 @@ extern "C" int bv_letterbox(bv_ctx *ctx, const uint8_t *const *srcs_host, const 
     BV_REQUIRE(ctx && srcs_host && heights_host && widths_host && out_dev, "null argument");
     BV_REQUIRE(n > 0 && n <= 65535 && out_h > 0 && out_w > 0 && out_h <= 65535, "bad batch or output size");
     BV_CUDA(cudaSetDevice(ctx->device));
+    // cv2.copyMakeBorder saturates the border value to uint8; the kernels index a 256-entry table with it
+    pad_value = pad_value < 0 ? 0 : (pad_value > 255 ? 255 : pad_value);
     static thread_local LetterboxImg descs[256];
     memset(descs, 0, sizeof(LetterboxImg) * (size_t)(n > 0 && n <= 256 ? n : 0));  // padding bytes compare equal
     BV_REQUIRE(n <= 256, "at most 256 images per call");
@@ -417,20 +419,32 @@ extern "C" int bv_letterbox(bv_ctx *ctx, const uint8_t *const *srcs_host, const 
         BV_CUDA(cudaMemcpyAsync(d_descs, descs, sizeof(LetterboxImg) * n, cudaMemcpyHostToDevice, ctx->stream));
         ctx->lb_cache_n = 0;  // the tap table is rebuilt below (or unused by the gather kernel)
     }
-    bool fits = true;  // the staged kernel holds two source rows in shared memory
+    bool fits = true;  // the staged kernel holds two source rows and the tap table in shared memory
     for (int i = 0; i < n; ++i) fits = fits && (size_t)widths_host[i] * 3 <= (size_t)kLbMaxRowBytes;
     static const bool use_tma = getenv("BV_LETTERBOX_GATHER") == nullptr;
-    if (fits && use_tma) {
-        const int n_items = out_h * n;
-        int max_w = 0;
-        for (int i = 0; i < n; ++i) max_w = widths_host[i] > max_w ? widths_host[i] : max_w;
-        const int row_stride = (max_w * 3 + 127) & ~127;
-        const size_t smem = (size_t)kLbStages * 2 * row_stride + sizeof(LbCoef) * (size_t)out_w;
-        if (smem > (size_t)ctx->lb_smem_set) {
+    int max_w = 0;
+    for (int i = 0; i < n; ++i) max_w = widths_host[i] > max_w ? widths_host[i] : max_w;
+    const int row_stride = (max_w * 3 + 127) & ~127;
+    const size_t smem = (size_t)kLbStages * 2 * row_stride + sizeof(LbCoef) * (size_t)out_w;
+    if (fits && use_tma && smem > (size_t)ctx->lb_smem_set) {
+        // the tap table grows with out_w: past the device's opt-in shared memory (out_w of ~24 000 on a
+        // B200) the gather kernel, which needs none, takes the call
+        int optin = 0;
+        BV_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+        cudaFuncAttributes fa16, fa32;
+        BV_CUDA(cudaFuncGetAttributes(&fa16, letterbox_tma_kernel<true>));
+        BV_CUDA(cudaFuncGetAttributes(&fa32, letterbox_tma_kernel<false>));
+        const size_t static_smem = fa16.sharedSizeBytes > fa32.sharedSizeBytes ? fa16.sharedSizeBytes : fa32.sharedSizeBytes;
+        if (smem + static_smem > (size_t)optin) {
+            fits = false;
+        } else {
             BV_CUDA(cudaFuncSetAttribute(letterbox_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             BV_CUDA(cudaFuncSetAttribute(letterbox_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             ctx->lb_smem_set = (int)smem;
         }
+    }
+    if (fits && use_tma) {
+        const int n_items = out_h * n;
         // persistent blocks: as many as fit next to each other (dynamic rows + ~14 KB of static tables)
         int per_sm = (int)((208 * 1024) / (smem + 6 * 1024));
         per_sm = per_sm < 1 ? 1 : (per_sm > 6 ? 6 : per_sm);

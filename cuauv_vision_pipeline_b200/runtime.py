@@ -345,15 +345,8 @@ class Context:
         return n, out
 
     def resize(self, src, width, height):
-        if src.dim() == 2:
-            b, sh, sw, c = 1, src.shape[0], src.shape[1], 1
-            shape = (height, width)
-        elif src.dim() == 3:
-            b, sh, sw, c = 1, src.shape[0], src.shape[1], src.shape[2]
-            shape = (height, width, c)
-        else:
-            b, sh, sw, c = src.shape
-            shape = (b, height, width, c)
+        b, sh, sw, c = self._bhw(src)
+        shape = (height, width) if src.dim() == 2 else ((height, width, c) if src.dim() == 3 else (b, height, width, c))
         dst = self.empty(shape)
         check(lib.bv_resize_linear(self.handle, _u8ptr(src), sh, sw, _u8ptr(dst), height, width, c, b))
         return dst
@@ -454,10 +447,17 @@ class Context:
         return dst
 
     def letterbox(self, images, out_h=640, out_w=640, pad=114, half=True, out=None):
+        """images: contiguous CUDA uint8 [H,W,3] BGR frames.  out: None, or a contiguous [n,3,out_h,out_w] fp16 (half) /
+        fp32 tensor on this context's device.  pad is saturated to 0..255."""
         n = len(images)
         for im in images:
-            if im.dim() != 3 or im.shape[2] != 3 or im.dtype != torch.uint8 or not im.is_cuda:
-                raise BVError(-1, "letterbox needs CUDA uint8 [H,W,3] tensors")
+            if im.dim() != 3 or im.shape[2] != 3 or im.dtype != torch.uint8 or not im.is_cuda or not im.is_contiguous():
+                raise BVError(-1, "letterbox needs contiguous CUDA uint8 [H,W,3] tensors")
+        if out is not None:
+            if (tuple(out.shape) != (n, 3, out_h, out_w) or out.dtype != (torch.float16 if half else torch.float32)
+                    or not out.is_contiguous() or out.device != self.device):
+                raise BVError(-1, "out= must be a contiguous %s [%d,3,%d,%d] tensor on %s"
+                              % ("float16" if half else "float32", n, out_h, out_w, self.device))
         srcs = ffi.new("uint8_t *[]", [_u8ptr(im) for im in images])
         hs = ffi.new("int32_t[]", [int(im.shape[0]) for im in images])
         ws = ffi.new("int32_t[]", [int(im.shape[1]) for im in images])

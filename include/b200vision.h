@@ -271,7 +271,8 @@ int bv_resize_linear(bv_ctx *ctx, const uint8_t *src_dev, int src_h, int src_w, 
                      int dst_w, int channels, int batch);
 /* Letterbox + BGR->RGB + HWC->CHW + /255 for n frames of possibly different sizes
  * (the Ultralytics pre-transform behind modules/yolo.py:112).  srcs_host: n device pointers;
- * out_dev: [n,3,out_h,out_w] of fp16 (out_fp16 != 0) or fp32. */
+ * out_dev: [n,3,out_h,out_w] of fp16 (out_fp16 != 0) or fp32.  n <= 256.  pad_value is saturated
+ * to 0..255 as cv2.copyMakeBorder does on uint8 (300 pads with 255, -5 with 0). */
 int bv_letterbox(bv_ctx *ctx, const uint8_t *const *srcs_host, const int32_t *heights_host,
                  const int32_t *widths_host, int n, void *out_dev, int out_h, int out_w, int pad_value,
                  int out_fp16);
