@@ -246,10 +246,20 @@ __global__ void __launch_bounds__(1024) ccl_scan_kernel(const int *__restrict__ 
     }
 }
 
-// one warp per row: number the roots of the row in raster order, store -(label) in parent[root]
+// bit `node` of frame f's frame-touching bitmap (bg_outer_kernel)
+__device__ __forceinline__ bool is_outer(const uint32_t *outer, int height, int width, size_t f, int node) {
+    const size_t words_per_frame = ((size_t)height * width + 31) / 32;
+    return (outer[f * words_per_frame + (node >> 5)] >> (node & 31)) & 1u;
+}
+
+// one warp per row: number the roots of the row in raster order, store -(label) in parent[root].  SKIP_OUTER: roots
+// marked in the frame-touching bitmap `outer` (bg_outer_kernel) are left alone and get no number (they keep parent[root]
+// == root)
+template <bool SKIP_OUTER>
 __global__ void __launch_bounds__(256) ccl_rank_kernel(const uint32_t *__restrict__ bits, int *__restrict__ parent,
                                                        const int *__restrict__ row_off, int height, int width, int wpr,
-                                                       size_t total_rows, int *__restrict__ root_px, int max_roots) {
+                                                       size_t total_rows, int *__restrict__ root_px, int max_roots,
+                                                       const uint32_t *__restrict__ outer) {
     const int lane = threadIdx.x & 31;
     const size_t warp0 = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const size_t nwarps = ((size_t)gridDim.x * blockDim.x) >> 5;
@@ -267,7 +277,8 @@ __global__ void __launch_bounds__(256) ccl_rank_kernel(const uint32_t *__restric
                 const int s = __ffs(s_it) - 1;
                 s_it &= s_it - 1;
                 const int node = y * width + wx * 32 + s;
-                if (fp[node] == node) roots |= 1u << s;
+                if (fp[node] == node && !(SKIP_OUTER && is_outer(outer, height, width, (row - y) / height, node)))
+                    roots |= 1u << s;
             }
             const int c = __popc(roots);
             int incl = c;
@@ -500,6 +511,39 @@ __global__ void __launch_bounds__(256, 4) ccl_final_kernel(const uint32_t *__res
     if (blobs) acc_flush(acc, blobs, max_blobs, carry_key, lane);
 }
 
+// node (pixel index of the run start) of the set pixel (y, x) in a bit image
+__device__ __forceinline__ int node_of(const uint32_t *frame_bits, int wpr, int width, int y, int x) {
+    const uint32_t w = frame_bits[(size_t)y * wpr + (x >> 5)];
+    return y * width + (x & ~31) + run_start(w, x & 31);
+}
+
+// mark the background regions that touch the image frame: outer[root >> 5] |= 1 << (root & 31).  UNCOUNT: also take
+// every newly marked root off its row's root count, so that the scan and rank steps number only the holes
+template <bool UNCOUNT>
+__global__ void __launch_bounds__(256) bg_outer_kernel(const uint32_t *__restrict__ inv, const int *__restrict__ parent,
+                                                       uint32_t *__restrict__ outer, int height, int width, int wpr,
+                                                       int batch, int *__restrict__ row_count) {
+    const int per_frame = 2 * width + 2 * height;
+    const size_t total = (size_t)per_frame * batch;
+    const size_t words_per_frame = ((size_t)height * width + 31) / 32;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int f = (int)(i / per_frame);
+        int k = (int)(i - (size_t)f * per_frame), x, y;
+        if (k < width) { y = 0; x = k; }
+        else if (k < 2 * width) { y = height - 1; x = k - width; }
+        else if (k < 2 * width + height) { x = 0; y = k - 2 * width; }
+        else { x = width - 1; y = k - 2 * width - height; }
+        const uint32_t *fb = inv + (size_t)f * height * wpr;
+        if (!((fb[(size_t)y * wpr + (x >> 5)] >> (x & 31)) & 1u)) continue;
+        const int *fp = parent + (size_t)f * height * width;
+        const int node = node_of(fb, wpr, width, y, x);
+        const int p = fp[node];
+        const int root = p;  // nodes were compressed to their root by ccl_count_kernel (roots point to themselves)
+        const uint32_t old = atomicOr(&outer[(size_t)f * words_per_frame + (root >> 5)], 1u << (root & 31));
+        if (UNCOUNT && !(old & (1u << (root & 31)))) atomicSub(&row_count[(size_t)f * height + root / width], 1);
+    }
+}
+
 // Scratch of the labelling for a batch of `batch` frames; frames f0.. of the batch use the slices at f0 (label_scratch_slice),
 // so that independent chunks of one batch can be labelled concurrently on different streams.
 int label_scratch(bv_ctx *ctx, int batch, int height, int width, LabelScratch *ls) {
@@ -523,7 +567,8 @@ static LabelScratch label_scratch_slice(const LabelScratch &ls, int f0, int heig
 }
 
 static int label_bits_ex(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int batch, int height, int width,
-                         bv_blob *blobs, int max_blobs, int32_t *n_blobs, int *root_px, int max_roots, const LabelScratch &sc);
+                         bv_blob *blobs, int max_blobs, int32_t *n_blobs, int *root_px, int max_roots, const LabelScratch &sc,
+                         uint32_t *outer = nullptr);
 
 int label_bits(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int batch, int height, int width, bv_blob *blobs,
                int max_blobs, int32_t *n_blobs) {
@@ -539,8 +584,13 @@ int label_bits_slice(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int f0,
                          label_scratch_slice(ls, f0, height, width));
 }
 
+// Foreground (`outer` == NULL): 8-connected components of `bits`.  Background (`outer` != NULL): `bits` is the inverted
+// mask and its regions are 4-connected (the background of an 8-connected foreground); the regions that touch the image
+// frame are marked in the bitmap `outer` (batch x ceil(H*W / 32) words) and, when `root_px` is given, the other regions
+// -- the holes -- are counted and numbered in raster order of their first pixel, frame-touching regions skipped.
 static int label_bits_ex(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int batch, int height, int width,
-                         bv_blob *blobs, int max_blobs, int32_t *n_blobs, int *root_px, int max_roots, const LabelScratch &sc) {
+                         bv_blob *blobs, int max_blobs, int32_t *n_blobs, int *root_px, int max_roots, const LabelScratch &sc,
+                         uint32_t *outer) {
     const int wpr = words_per_row(width);
     const size_t total_words = (size_t)batch * height * wpr;
     const size_t total_rows = (size_t)batch * height;
@@ -555,10 +605,27 @@ static int label_bits_ex(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int
     const int gw = grid_for(ctx, total_words, 256, 8);
     const int gr = grid_for(ctx, total_rows * 32, 256, 8);
     BV_LAUNCH(ctx, ccl_init_kernel, gw, 256, 0, bits, parent, height, width, wpr, (uint32_t)total_words);
+    if (outer) {
+        const bool holes = root_px != nullptr;
+        BV_LAUNCH(ctx, ccl_merge_kernel<false>, gw, 256, 0, bits, parent, height, width, wpr, (uint32_t)total_words);
+        BV_LAUNCH(ctx, ccl_count_kernel, gr, 256, 0, bits, parent, row_count, height, width, wpr, total_rows);
+        BV_CUDA(cudaMemsetAsync(outer, 0, (size_t)batch * (((size_t)height * width + 31) / 32) * 4, ctx->stream));
+        const int ge = grid_for(ctx, (size_t)batch * (2 * width + 2 * height), 256, 8);
+        if (!holes) {
+            BV_LAUNCH(ctx, bg_outer_kernel<false>, ge, 256, 0, bits, parent, outer, height, width, wpr, batch, nullptr);
+            return BV_OK;
+        }
+        BV_LAUNCH(ctx, bg_outer_kernel<true>, ge, 256, 0, bits, parent, outer, height, width, wpr, batch, row_count);
+        BV_LAUNCH(ctx, ccl_scan_kernel, batch, 1024, 0, row_count, row_off, nb, height, nullptr, 0, width);
+        BV_LAUNCH(ctx, ccl_rank_kernel<true>, gr, 256, 0, bits, parent, row_off, height, width, wpr, total_rows, root_px,
+                  max_roots, outer);
+        return BV_OK;
+    }
     BV_LAUNCH(ctx, ccl_merge_kernel<true>, gw, 256, 0, bits, parent, height, width, wpr, (uint32_t)total_words);
     BV_LAUNCH(ctx, ccl_count_kernel, gr, 256, 0, bits, parent, row_count, height, width, wpr, total_rows);
     BV_LAUNCH(ctx, ccl_scan_kernel, batch, 1024, 0, row_count, row_off, nb, height, (max_blobs > 0 ? blobs : nullptr), max_blobs, width);
-    BV_LAUNCH(ctx, ccl_rank_kernel, gr, 256, 0, bits, parent, row_off, height, width, wpr, total_rows, root_px, max_roots);
+    BV_LAUNCH(ctx, ccl_rank_kernel<false>, gr, 256, 0, bits, parent, row_off, height, width, wpr, total_rows, root_px, max_roots,
+              nullptr);
     if (labels || (blobs && max_blobs > 0))
         BV_LAUNCH(ctx, ccl_final_kernel, gw, 256, 0, bits, parent, labels, (max_blobs > 0 ? blobs : nullptr), max_blobs,
                   height, width, wpr, (uint32_t)total_words);
@@ -580,6 +647,12 @@ static int label_bits_ex(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int
 //    neighbour, then counter-clockwise from the direction it came from) and accumulates
 //    a00 = sum(x' y - x y'), a10 = sum(dxy (x' + x)), a01 = sum(dxy (y' + y)) in int64: exact, and
 //    independent of CHAIN_APPROX_SIMPLE (collinear points split a term into equal parts).
+//
+// Hole borders and the hierarchy (bv_find_contours, RETR_LIST / CCOMP / TREE): the background
+// regions that do not reach the frame are the holes; the same count / scan / rank steps number
+// them in raster order of their first pixel.  A hole border starts at the pixel left of the hole's
+// first pixel and is followed by the same walk; the hole that encloses an outer border is the one
+// left of its start pixel, and the component that encloses a hole border owns its start pixel.
 // ----------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) invert_bits_kernel(const uint32_t *__restrict__ src, uint32_t *__restrict__ dst,
                                                           int width, int wpr, uint32_t total_words) {
@@ -590,36 +663,6 @@ __global__ void __launch_bounds__(256) invert_bits_kernel(const uint32_t *__rest
         uint32_t w = ~src[i];
         if ((int)(i % (uint32_t)wpr) == wpr - 1) w &= tail_mask;
         dst[i] = w;
-    }
-}
-
-// node (pixel index of the run start) of the set pixel (y, x) in a bit image
-__device__ __forceinline__ int node_of(const uint32_t *frame_bits, int wpr, int width, int y, int x) {
-    const uint32_t w = frame_bits[(size_t)y * wpr + (x >> 5)];
-    return y * width + (x & ~31) + run_start(w, x & 31);
-}
-
-// mark the background regions that touch the image frame: outer[root >> 5] |= 1 << (root & 31)
-__global__ void __launch_bounds__(256) bg_outer_kernel(const uint32_t *__restrict__ inv, const int *__restrict__ parent,
-                                                       uint32_t *__restrict__ outer, int height, int width, int wpr,
-                                                       int batch) {
-    const int per_frame = 2 * width + 2 * height;
-    const size_t total = (size_t)per_frame * batch;
-    const size_t words_per_frame = ((size_t)height * width + 31) / 32;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-        const int f = (int)(i / per_frame);
-        int k = (int)(i - (size_t)f * per_frame), x, y;
-        if (k < width) { y = 0; x = k; }
-        else if (k < 2 * width) { y = height - 1; x = k - width; }
-        else if (k < 2 * width + height) { x = 0; y = k - 2 * width; }
-        else { x = width - 1; y = k - 2 * width - height; }
-        const uint32_t *fb = inv + (size_t)f * height * wpr;
-        if (!((fb[(size_t)y * wpr + (x >> 5)] >> (x & 31)) & 1u)) continue;
-        const int *fp = parent + (size_t)f * height * width;
-        const int node = node_of(fb, wpr, width, y, x);
-        const int p = fp[node];
-        const int root = p;  // nodes were compressed to their root by ccl_count_kernel (roots point to themselves)
-        atomicOr(&outer[(size_t)f * words_per_frame + (root >> 5)], 1u << (root & 31));
     }
 }
 
@@ -668,17 +711,46 @@ constexpr int kChunkPoints = 31;                  // vertices per chunk
 constexpr int kChunkInts = 2 * kChunkPoints + 2;  // + index of the next chunk + padding = 256 bytes
 constexpr int kChunksOverflowed = -2;             // the pool ran dry under this border: it is walked again
 
-// WRITE = false: first walk (sums, counts, externality).  WRITE = true: second walk of the external
-// borders that got a slot in the point list, emitting the CHAIN_APPROX_SIMPLE vertices.
-template <bool WRITE>
+// What the walk needs besides the RETR_EXTERNAL inputs when it serves bv_find_contours (TREE = true): records
+// 0 .. n_outer-1 are the outer borders, as for RETR_EXTERNAL, and the hole borders follow them.
+struct TreeArgs {
+    const int *n_holes;       // [batch] holes per frame (ranked background labelling)
+    const int *hole_px;       // [batch][max_contours] first pixel of every hole, raster order
+    const uint32_t *fg_bits;  // the foreground mask, row-major words
+    const int *fg_parent;     // the ranked foreground union-find: parent[root] = -label, other nodes point at their root
+    int *enclosing;           // [batch][max_contours] out: outer border -> hole index or -1, hole border -> label - 1
+    int none;                 // CHAIN_APPROX_NONE: every border pixel is a vertex
+};
+
+// hole index of the background pixel (x, y) once the holes are ranked (ccl_rank_kernel<true>); -1 for a frame-touching
+// region, whose root keeps parent[root] == root
+__device__ __forceinline__ int hole_of(const uint32_t *frame_inv, const int *frame_parent, int wpr, int width, int y, int x) {
+    const int v = frame_parent[node_of(frame_inv, wpr, width, y, x)];
+    if (v < 0) return -v - 1;
+    const int r = frame_parent[v];
+    return r < 0 ? -r - 1 : -1;
+}
+
+// records of frame f that the walk writes
+template <bool TREE>
+__device__ __forceinline__ int records_of(const int *n_blobs, const int *n_holes, int f, int max_contours) {
+    if (!TREE) return min(n_blobs[f], max_contours);
+    return (int)min((long long)n_blobs[f] + n_holes[f], (long long)max_contours);
+}
+
+// WRITE = false: first walk (sums, counts, externality).  WRITE = true: second walk of the borders that got a slot in
+// the point list but whose vertices the pool could not hold.  TREE = false: the external borders' CHAIN_APPROX_SIMPLE
+// vertices (bv_outer_contours); TREE = true: outer and hole borders, CHAIN_APPROX_SIMPLE or NONE (bv_find_contours).
+template <bool WRITE, bool TREE>
 __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict__ bits, const uint32_t *__restrict__ inv,
                                                       const int *__restrict__ parent_bg, const uint32_t *__restrict__ outer,
                                                       const int *__restrict__ root_px, const int *__restrict__ n_blobs,
                                                       bv_contour *__restrict__ out, int max_contours, int height, int width,
                                                       int wpr, int wcols, int *__restrict__ points, int max_points, int lane_stride,
-                                                      int *__restrict__ pool, int *__restrict__ pool_next, int pool_chunks) {
+                                                      int *__restrict__ pool, int *__restrict__ pool_next, int pool_chunks,
+                                                      TreeArgs ta) {
     const int f = blockIdx.y;
-    const int n = min(n_blobs[f], max_contours);
+    const int n = records_of<TREE>(n_blobs, ta.n_holes, f, max_contours);
     // one border per thread, but only every fourth lane takes one: a warp-wide load of 32 walks touches 32 different
     // lines and every step waits for the slowest of them
     if (threadIdx.x % lane_stride) return;
@@ -686,15 +758,30 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
     if (idx >= n) return;
     const unsigned rows = (unsigned)height + 2;
     const uint32_t *fw = bits + (size_t)f * wcols * rows;  // walk_bits_kernel's copy
+    // a hole border starts at the pixel left of the hole's first pixel, and cv2 starts its clockwise search there from E
+    // (from W for an outer border)
+    const bool hole = TREE && idx >= n_blobs[f];
+    const bool none = TREE && ta.none;
     bv_contour c;
     int *pts = nullptr;
     int x0, y0;
     if (WRITE) {
         c = out[(size_t)f * max_contours + idx];
-        if (!c.external || c.point_offset < 0 || c.reserved != kChunksOverflowed) return;  // the gather kernel served the rest
+        if ((!TREE && !c.external) || c.point_offset < 0 || c.reserved != kChunksOverflowed) return;  // the gather kernel served the rest
         pts = points + ((size_t)f * max_points + c.point_offset) * 2;
         x0 = c.start_x;
         y0 = c.start_y;
+    } else if (hole) {
+        const int start = ta.hole_px[(size_t)f * max_contours + idx - n_blobs[f]];
+        y0 = start / width;
+        x0 = start - y0 * width - 1;  // foreground: the hole does not reach the frame
+        const int *fp = ta.fg_parent + (size_t)f * height * width;
+        const int v = fp[node_of(ta.fg_bits + (size_t)f * height * wpr, wpr, width, y0, x0)];
+        c.label = v < 0 ? -v : -fp[v];
+        c.start_x = x0;
+        c.start_y = y0;
+        c.external = 0;
+        ta.enclosing[(size_t)f * max_contours + idx] = c.label - 1;
     } else {
         const int start = root_px[(size_t)f * max_contours + idx];
         y0 = start / width;
@@ -704,7 +791,13 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
         c.start_y = y0;
         // external iff the background on the left reaches the frame (or the start pixel is on the frame)
         int external = 1;
-        if (x0 > 0) {
+        if (TREE) {
+            const int h = x0 > 0 ? hole_of(inv + (size_t)f * height * wpr, parent_bg + (size_t)f * height * width, wpr,
+                                           width, y0, x0 - 1)
+                                 : -1;
+            external = h < 0;
+            ta.enclosing[(size_t)f * max_contours + idx] = h;
+        } else if (x0 > 0) {
             const uint32_t *fi = inv + (size_t)f * height * wpr;
             const int node = node_of(fi, wpr, width, y0, x0 - 1);
             const int root = parent_bg[(size_t)f * height * width + node];
@@ -720,9 +813,9 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
 #define dy(s) ((int)((0x22210001u >> (4 * (s))) & 0xFu) - 1)
     long long a00 = 0, a10 = 0, a01 = 0;
     int bx0 = x0, bx1 = x0, by0 = y0, by1 = y0, npts = 1, nsimple = 1;
-    // first walk of an external border: its vertices also go into a chain of 31-point chunks drawn from the frame's
-    // pool, so that they need not be found again by a second walk once the offsets in the point list are known
-    const bool store = !WRITE && pool != nullptr && c.external;
+    // first walk of a border whose vertices are wanted: they also go into a chain of 31-point chunks drawn from the
+    // frame's pool, so that they need not be found again by a second walk once the offsets in the point list are known
+    const bool store = !WRITE && pool != nullptr && (TREE || c.external);
     int *fpool = store ? pool + (size_t)f * pool_chunks * kChunkInts : nullptr;
     int first_chunk = -1, chunk = -1, slot = kChunkPoints;
     auto keep_vertex = [&](int vx, int vy) {
@@ -741,10 +834,10 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
         fpool[(size_t)chunk * kChunkInts + 2 * slot + 1] = vy;
         ++slot;
     };
-    int s = 4;
+    int s = hole ? 0 : 4;
     bool found = false;
     const uint32_t nb0 = neighbours_at(fw, rows, x0, y0);
-    for (int k = 0; k < 7; ++k) {  // clockwise from W: NW, N, NE, E, SE, S, SW
+    for (int k = 0; k < 7; ++k) {  // clockwise from W: NW, N, NE, E, SE, S, SW (from E: SE, S, SW, W, NW, N, NE)
         s = (s - 1) & 7;
         if ((nb0 >> s) & 1u) {
             found = true;
@@ -760,7 +853,10 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
     } else {
         const int x1 = x0 + dx(s), y1 = y0 + dy(s);  // i1: the first neighbour, where the walk will end
         int cx = x0, cy = y0;                        // i3
-        int prev_s = s ^ 4;                          // CHAIN_APPROX_SIMPLE: keep a point when the direction turns
+        // CHAIN_APPROX_SIMPLE: keep a point when the direction turns.  The walk ends with the step i1 -> i0, in direction
+        // s ^ 4, so the start pixel is kept iff the chain turns there, as CHAIN_APPROX_SIMPLE treats it: always for an
+        // outer border (its start is the component's first pixel), not always for a hole border.
+        int prev_s = s ^ 4;
         npts = 0;
         nsimple = 0;
         for (;;) {
@@ -772,12 +868,16 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
             s = (first + __ffs(((nb | (nb << 8)) >> first) & 0xFFu) - 1) & 7;
             const int ddx = dx(s), ddy = dy(s);
             const int nx = cx + ddx, ny = cy + ddy;
-            if (s != prev_s) {
+            const bool turn = s != prev_s;
+            if (turn || none) {
                 if (WRITE) {
-                    pts[2 * nsimple] = cx;
-                    pts[2 * nsimple + 1] = cy;
+                    const int k = none ? npts : nsimple;
+                    pts[2 * k] = cx;
+                    pts[2 * k + 1] = cy;
                 }
                 keep_vertex(cx, cy);
+            }
+            if (turn) {
                 ++nsimple;
                 prev_s = s;
             }
@@ -814,21 +914,23 @@ __global__ void __launch_bounds__(128) contour_kernel(const uint32_t *__restrict
     out[(size_t)f * max_contours + idx] = c;
 }
 
-// one block per frame: hand every external contour its slice of the frame's point list
-// (exclusive scan of n_simple in raster order; sequential over chunks of blockDim contours)
+// one block per frame: hand every border that lists its vertices (the external ones; TREE: all) its slice of the frame's
+// point list (exclusive scan of the vertex counts in record order; sequential over chunks of blockDim contours)
+template <bool TREE>
 __global__ void __launch_bounds__(1024) contour_offsets_kernel(bv_contour *__restrict__ contours, const int *__restrict__ n_blobs,
-                                                               int max_contours, int max_points, int *__restrict__ n_points) {
+                                                               int max_contours, int max_points, int *__restrict__ n_points,
+                                                               const int *__restrict__ n_holes, int none) {
     __shared__ int warp_sums[32];
     __shared__ int carry;
     const int f = blockIdx.x;
-    const int n = min(n_blobs[f], max_contours);
+    const int n = records_of<TREE>(n_blobs, n_holes, f, max_contours);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     bv_contour *fc = contours + (size_t)f * max_contours;
     if (threadIdx.x == 0) carry = 0;
     __syncthreads();
     for (int base = 0; base < n; base += blockDim.x) {
         const int i = base + threadIdx.x;
-        const int v = (i < n && fc[i].external) ? fc[i].n_simple : 0;
+        const int v = (i < n && (TREE || fc[i].external)) ? (TREE && none ? fc[i].n_points : fc[i].n_simple) : 0;
         int incl = v;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
@@ -856,18 +958,20 @@ __global__ void __launch_bounds__(1024) contour_offsets_kernel(bv_contour *__res
     if (threadIdx.x == 0 && n_points) n_points[f] = carry;
 }
 
-// One warp per external contour that got a slice of the point list: copies its chain of chunks into the slice.
+// One warp per listed contour that got a slice of the point list: copies its chain of chunks into the slice.
+template <bool TREE>
 __global__ void __launch_bounds__(128) contour_gather_kernel(bv_contour *__restrict__ contours, const int *__restrict__ n_blobs,
                                                              int max_contours, const int *__restrict__ pool, int pool_chunks,
-                                                             int *__restrict__ points, int max_points) {
+                                                             int *__restrict__ points, int max_points,
+                                                             const int *__restrict__ n_holes, int none) {
     const int f = blockIdx.y;
-    const int n = min(n_blobs[f], max_contours);
+    const int n = records_of<TREE>(n_blobs, n_holes, f, max_contours);
     const int lane = threadIdx.x & 31;
     const int idx = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (idx >= n) return;
     bv_contour *c = contours + (size_t)f * max_contours + idx;
-    const int first = c->reserved, offset = c->point_offset, count = c->n_simple;
-    if (!c->external) return;
+    const int first = c->reserved, offset = c->point_offset, count = (TREE && none) ? c->n_points : c->n_simple;
+    if (!TREE && !c->external) return;
     __syncwarp();
     if (first == kChunksOverflowed && offset >= 0) return;    // keeps the mark: the second walk writes its vertices
     if (lane == 0) c->reserved = 0;
@@ -883,8 +987,67 @@ __global__ void __launch_bounds__(128) contour_gather_kernel(bv_contour *__restr
     }
 }
 
-int outer_contours_bits(bv_ctx *ctx, const uint32_t *bits, int batch, int height, int width, bv_contour *contours,
-                        int max_contours, int32_t *n_contours, int32_t *points, int max_points, int32_t *n_points) {
+// One block per frame: cv2's hierarchy rows (next, prev, first_child, parent) of the records the walk wrote, and the
+// frame's two counts.  Parents follow from `enclosing` and the mode; siblings are the records with the same parent, linked
+// in increasing record order.  `next` comes from one warp that runs over the records from the last to the first, 32 at a
+// time, keeping head[parent + 1] = the smallest record seen so far with that parent; `prev` is its inverse and
+// first_child[p] is head[p + 1] at the end.  No atomics: the result does not depend on scheduling.
+__global__ void __launch_bounds__(1024) contour_tree_kernel(int *__restrict__ enclosing, const int *__restrict__ n_outer_of,
+                                                            const int *__restrict__ n_holes_of, int max_contours, int mode,
+                                                            int4 *__restrict__ hierarchy, int *__restrict__ n_contours,
+                                                            int *head_global) {
+    extern __shared__ int head_shared[];
+    const int f = blockIdx.x;
+    const int n_outer = n_outer_of[f];
+    const int n = records_of<true>(n_outer_of, n_holes_of, f, max_contours);
+    int *par = enclosing + (size_t)f * max_contours;
+    int4 *hier = hierarchy + (size_t)f * max_contours;
+    int *head = head_global ? head_global + (size_t)f * (max_contours + 1) : head_shared;  // head[0]: parent -1
+    if (threadIdx.x == 0 && n_contours) {
+        n_contours[2 * f] = n_outer;
+        n_contours[2 * f + 1] = n_holes_of[f];
+    }
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const int e = par[i];
+        int p = -1;
+        if (i >= n_outer)
+            p = mode == BV_RETR_LIST ? -1 : e;                            // hole -> its component's outer border
+        else if (mode == BV_RETR_TREE && e >= 0 && n_outer + e < n)
+            p = n_outer + e;                                              // outer border -> the hole around it
+        par[i] = p;
+        hier[i] = make_int4(-1, -1, -1, p);
+    }
+    for (int k = threadIdx.x; k <= n; k += blockDim.x) head[k] = -1;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        const int lane = threadIdx.x;
+        for (int base = (n - 1) & ~31; base >= 0; base -= 32) {
+            const int i = base + lane;
+            const bool valid = i < n;
+            const int key = valid ? par[i] + 1 : -1 - lane;               // invalid lanes match nobody
+            const unsigned peers = __match_any_sync(0xFFFFFFFFu, key);
+            const unsigned later = peers & ~((2u << lane) - 1u);
+            const int next = !valid ? -1 : later ? base + __ffs(later) - 1 : head[key];
+            __syncwarp();
+            if (valid && !(peers & ((1u << lane) - 1u))) head[key] = i;   // the group's first record
+            if (valid) {
+                hier[i].x = next;
+                if (next >= 0) hier[next].y = i;
+            }
+            __syncwarp();
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < n; i += blockDim.x) hier[i].z = head[i + 1];
+}
+
+// RETR_EXTERNAL (mode < 0, bv_outer_contours): the outer borders, the external ones with their CHAIN_APPROX_SIMPLE
+// vertices, n_contours[batch].  RETR_LIST / CCOMP / TREE (bv_find_contours): the outer borders, then the hole borders,
+// all with vertices, n_contours[batch][2], and the hierarchy.
+static int contours_bits(bv_ctx *ctx, const uint32_t *bits, int batch, int height, int width, bv_contour *contours,
+                         int max_contours, int32_t *n_contours, int32_t *points, int max_points, int32_t *n_points, int mode,
+                         int none, int32_t *hierarchy) {
+    const bool tree = mode >= 0;
     const int wpr = words_per_row(width);
     const size_t total_words = (size_t)batch * height * wpr;
     const size_t total_rows = (size_t)batch * height;
@@ -893,28 +1056,36 @@ int outer_contours_bits(bv_ctx *ctx, const uint32_t *bits, int batch, int height
     BV_TRY(ensure_scratch(ctx, SCR_CCL_ROOTS, (size_t)batch * max_contours * sizeof(int)));
     BV_TRY(ensure_scratch(ctx, SCR_BITS_B, total_words * 8));
     BV_TRY(ensure_scratch(ctx, SCR_CCL_PARENT2, total_rows * width * sizeof(int)));
-    BV_TRY(ensure_scratch(ctx, SCR_CCL_AUX2, (total_rows + (size_t)batch * outer_words) * sizeof(int)));
+    BV_TRY(ensure_scratch(ctx, SCR_CCL_AUX2, (total_rows * 2 + batch + (size_t)batch * outer_words) * sizeof(int)));
     int *root_px = (int *)ctx->scratch[SCR_CCL_ROOTS];
     uint32_t *inv = (uint32_t *)ctx->scratch[SCR_BITS_B];
-    int *parent_bg = (int *)ctx->scratch[SCR_CCL_PARENT2];
-    int *row_count_bg = (int *)ctx->scratch[SCR_CCL_AUX2];
-    uint32_t *outer = (uint32_t *)(row_count_bg + total_rows);
+    LabelScratch bg;
+    bg.parent = (int *)ctx->scratch[SCR_CCL_PARENT2];
+    bg.row_count = (int *)ctx->scratch[SCR_CCL_AUX2];
+    bg.row_off = bg.row_count + total_rows;
+    bg.n_fallback = bg.row_off + total_rows;          // the hole count per frame
+    uint32_t *outer = (uint32_t *)(bg.n_fallback + batch);
+    // RETR_LIST / CCOMP / TREE: first pixel of every hole, the records' enclosing regions, the hierarchy's head table
+    int *hole_px = nullptr, *enclosing = nullptr, *head_global = nullptr;
+    const size_t head_bytes = ((size_t)max_contours + 1) * sizeof(int);
+    const bool head_in_smem = head_bytes <= 48 * 1024;
+    if (tree) {
+        BV_TRY(ensure_scratch(ctx, SCR_CCL_TREE, (size_t)batch * (2 * (size_t)max_contours + (head_in_smem ? 0 : max_contours + 1)) *
+                                                     sizeof(int)));
+        hole_px = (int *)ctx->scratch[SCR_CCL_TREE];
+        enclosing = hole_px + (size_t)batch * max_contours;
+        if (!head_in_smem) head_global = enclosing + (size_t)batch * max_contours;
+    }
     // foreground: labels are not needed, only the roots in raster order
     LabelScratch ls;
     BV_TRY(label_scratch(ctx, batch, height, width, &ls));
-    BV_TRY(label_bits_ex(ctx, bits, nullptr, batch, height, width, nullptr, 0, n_contours, root_px, max_contours, ls));
+    // label_bits_ex writes the blob count to n_blobs (its own scratch when NULL)
+    int *nb = tree ? ls.n_fallback : (n_contours ? n_contours : ls.n_fallback);
+    BV_TRY(label_bits_ex(ctx, bits, nullptr, batch, height, width, nullptr, 0, nb, root_px, max_contours, ls));
     // background, 4-connected
     const int gw = grid_for(ctx, total_words, 256, 8);
-    const int gr = grid_for(ctx, total_rows * 32, 256, 8);
     BV_LAUNCH(ctx, invert_bits_kernel, gw, 256, 0, bits, inv, width, wpr, (uint32_t)total_words);
-    BV_LAUNCH(ctx, ccl_init_kernel, gw, 256, 0, inv, parent_bg, height, width, wpr, (uint32_t)total_words);
-    BV_LAUNCH(ctx, ccl_merge_kernel<false>, gw, 256, 0, inv, parent_bg, height, width, wpr, (uint32_t)total_words);
-    BV_LAUNCH(ctx, ccl_count_kernel, gr, 256, 0, inv, parent_bg, row_count_bg, height, width, wpr, total_rows);
-    BV_CUDA(cudaMemsetAsync(outer, 0, (size_t)batch * outer_words * 4, ctx->stream));
-    BV_LAUNCH(ctx, bg_outer_kernel, grid_for(ctx, (size_t)batch * (2 * width + 2 * height), 256, 8), 256, 0, inv, parent_bg,
-              outer, height, width, wpr, batch);
-    // label_bits_ex wrote the blob count to n_contours (or its own scratch when NULL)
-    const int *nb = n_contours ? n_contours : (int *)ctx->scratch[SCR_CCL_AUX] + 2 * total_rows;
+    BV_TRY(label_bits_ex(ctx, inv, nullptr, batch, height, width, nullptr, 0, bg.n_fallback, hole_px, max_contours, bg, outer));
     const int wcols = (width + (int)kWalkPixelsPerWord - 1) / (int)kWalkPixelsPerWord;
     const size_t walk_words = (size_t)batch * wcols * (height + 2);
     BV_REQUIRE(walk_words < 0xFFFFFFFFull, "frames too large for the contour walk");
@@ -936,15 +1107,39 @@ int outer_contours_bits(bv_ctx *ctx, const uint32_t *bits, int batch, int height
         pool_next = pool + (size_t)batch * pool_chunks * kChunkInts;
         BV_CUDA(cudaMemsetAsync(pool_next, 0, batch * sizeof(int), ctx->stream));
     }
-    BV_LAUNCH(ctx, contour_kernel<false>, grid, 128, 0, walk, inv, parent_bg, outer, root_px, nb, contours, max_contours,
-              height, width, wpr, wcols, nullptr, 0, lane_stride, pool, pool_next, pool_chunks);
+    const TreeArgs ta = tree ? TreeArgs{bg.n_fallback, hole_px, bits, ls.parent, enclosing, none} : TreeArgs{};
+    const int *nh = ta.n_holes;
+    if (tree) {
+        BV_LAUNCH(ctx, (contour_kernel<false, true>), grid, 128, 0, walk, inv, bg.parent, outer, root_px, nb, contours,
+                  max_contours, height, width, wpr, wcols, nullptr, 0, lane_stride, pool, pool_next, pool_chunks, ta);
+    } else {
+        BV_LAUNCH(ctx, (contour_kernel<false, false>), grid, 128, 0, walk, inv, bg.parent, outer, root_px, nb, contours,
+                  max_contours, height, width, wpr, wcols, nullptr, 0, lane_stride, pool, pool_next, pool_chunks, ta);
+    }
     if (want_points) {
-        BV_LAUNCH(ctx, contour_offsets_kernel, batch, 1024, 0, contours, nb, max_contours, max_points, n_points);
-        BV_LAUNCH(ctx, contour_gather_kernel, dim3((max_contours + 3) / 4, batch), 128, 0, contours, nb, max_contours, pool,
-                  pool_chunks, points, max_points);
-        // borders the pool could not hold (it is sized so that this needs more vertices than max_points): walked again
-        BV_LAUNCH(ctx, contour_kernel<true>, grid, 128, 0, walk, inv, parent_bg, outer, root_px, nb, contours, max_contours,
-                  height, width, wpr, wcols, points, max_points, lane_stride, nullptr, nullptr, 0);
+        const dim3 gg((max_contours + 3) / 4, batch);
+        if (tree) {
+            BV_LAUNCH(ctx, contour_offsets_kernel<true>, batch, 1024, 0, contours, nb, max_contours, max_points, n_points, nh, none);
+            BV_LAUNCH(ctx, contour_gather_kernel<true>, gg, 128, 0, contours, nb, max_contours, pool, pool_chunks, points,
+                      max_points, nh, none);
+            BV_LAUNCH(ctx, (contour_kernel<true, true>), grid, 128, 0, walk, inv, bg.parent, outer, root_px, nb, contours,
+                      max_contours, height, width, wpr, wcols, points, max_points, lane_stride, nullptr, nullptr, 0, ta);
+        } else {
+            BV_LAUNCH(ctx, contour_offsets_kernel<false>, batch, 1024, 0, contours, nb, max_contours, max_points, n_points, nh, 0);
+            BV_LAUNCH(ctx, contour_gather_kernel<false>, gg, 128, 0, contours, nb, max_contours, pool, pool_chunks, points,
+                      max_points, nh, 0);
+            // borders the pool could not hold (it is sized so that this needs more vertices than max_points): walked again
+            BV_LAUNCH(ctx, (contour_kernel<true, false>), grid, 128, 0, walk, inv, bg.parent, outer, root_px, nb, contours,
+                      max_contours, height, width, wpr, wcols, points, max_points, lane_stride, nullptr, nullptr, 0, ta);
+        }
+    }
+    if (tree && (hierarchy || n_contours)) {
+        if (!hierarchy) {
+            BV_TRY(ensure_scratch(ctx, SCR_CCL_TREE_ROWS, (size_t)batch * max_contours * sizeof(int4)));
+            hierarchy = (int32_t *)ctx->scratch[SCR_CCL_TREE_ROWS];
+        }
+        BV_LAUNCH(ctx, contour_tree_kernel, batch, 1024, head_in_smem ? head_bytes : 0, enclosing, nb, nh, max_contours, mode,
+                  reinterpret_cast<int4 *>(hierarchy), n_contours, head_global);
     }
     return BV_OK;
 }
@@ -976,6 +1171,26 @@ extern "C" int bv_outer_contours(bv_ctx *ctx, const uint8_t *mask_dev, int batch
     BV_TRY(ensure_scratch(ctx, SCR_BITS_A, words * 4));
     uint32_t *bits = (uint32_t *)ctx->scratch[SCR_BITS_A];
     BV_TRY(mask_to_bits(ctx, mask_dev, bits, batch, height, width));
-    return outer_contours_bits(ctx, bits, batch, height, width, contours_dev, max_contours, n_contours_dev, points_dev,
-                               points_dev ? max_points : 0, n_points_dev);
+    return contours_bits(ctx, bits, batch, height, width, contours_dev, max_contours, n_contours_dev, points_dev,
+                         points_dev ? max_points : 0, n_points_dev, -1, 0, nullptr);
+}
+
+extern "C" int bv_find_contours(bv_ctx *ctx, const uint8_t *mask_dev, int batch, int height, int width, int mode, int method,
+                                bv_contour *contours_dev, int32_t *hierarchy_dev, int max_contours, int32_t *n_contours_dev,
+                                int32_t *points_dev, int max_points, int32_t *n_points_dev) {
+    BV_REQUIRE(ctx && mask_dev && contours_dev, "null argument");
+    BV_REQUIRE(batch > 0 && height > 0 && width > 0 && max_contours > 0, "sizes must be positive");
+    BV_REQUIRE(mode == BV_RETR_LIST || mode == BV_RETR_CCOMP || mode == BV_RETR_TREE,
+               "mode must be BV_RETR_LIST, BV_RETR_CCOMP or BV_RETR_TREE (RETR_EXTERNAL: bv_outer_contours)");
+    BV_REQUIRE(method == BV_CHAIN_APPROX_NONE || method == BV_CHAIN_APPROX_SIMPLE,
+               "method must be BV_CHAIN_APPROX_NONE or BV_CHAIN_APPROX_SIMPLE");
+    BV_REQUIRE(max_points >= 0, "max_points must be >= 0");
+    BV_REQUIRE(((uintptr_t)hierarchy_dev & 15) == 0, "hierarchy_dev must be 16-byte aligned");
+    BV_CUDA(cudaSetDevice(ctx->device));
+    const size_t words = (size_t)batch * bits_frame_words(height, width);
+    BV_TRY(ensure_scratch(ctx, SCR_BITS_A, words * 4));
+    uint32_t *bits = (uint32_t *)ctx->scratch[SCR_BITS_A];
+    BV_TRY(mask_to_bits(ctx, mask_dev, bits, batch, height, width));
+    return contours_bits(ctx, bits, batch, height, width, contours_dev, max_contours, n_contours_dev, points_dev,
+                         points_dev ? max_points : 0, n_points_dev, mode, method == BV_CHAIN_APPROX_NONE, hierarchy_dev);
 }

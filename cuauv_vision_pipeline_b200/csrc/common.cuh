@@ -87,8 +87,10 @@ enum ScratchSlot {
     SCR_CCL_PARENT,     // union-find parents, int32 per pixel
     SCR_CCL_AUX,        // per-block root counts / offsets
     SCR_CCL_PARENT2,    // union-find parents of the background regions (outer contours)
-    SCR_CCL_AUX2,       // background row counts + frame-touching bitmap
+    SCR_CCL_AUX2,       // background row counts / offsets, hole counts, frame-touching bitmap
     SCR_CCL_ROOTS,      // first pixel of every blob, raster order
+    SCR_CCL_TREE,       // first pixel of every hole, enclosing region of every border, hierarchy head table (find_contours)
+    SCR_CCL_TREE_ROWS,  // hierarchy rows when the caller passes none
     SCR_HULL,           // sorted vertices + hull stack per contour (minAreaRect)
     SCR_NOISE_RAW,      // raw MT19937 words replayed for the Gaussian-noise step
     SCR_NOISE_AUX,      // per-block accepted counts / offsets of the polar method

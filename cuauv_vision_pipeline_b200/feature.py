@@ -30,7 +30,8 @@ def label_blobs(mat, max_blobs=4096, want_labels=True):
 
 
 class Contour(dict):
-    """One outer border (cv2.findContours RETR_EXTERNAL) reduced to its Green's-theorem sums."""
+    """One border of cv2.findContours reduced to its Green's-theorem sums (the fields of bv_contour), with its vertices
+    where they were asked for."""
 
 
 def outer_contours(mat, max_contours=4096, points=False, max_points=None, rects=False):
@@ -66,6 +67,60 @@ def outer_contours(mat, max_contours=4096, points=False, max_points=None, rects=
             off = c["point_offset"]
             c["points"] = host[off:off + c["n_simple"]].reshape(-1, 1, 2).copy() if off >= 0 else None
     return out
+
+
+def find_contours(mat, mode="tree", method="simple", max_contours=4096, max_points=None):
+    """cv2.findContours(mat, RETR_<mode>, CHAIN_APPROX_<method>) on the GPU for one mask: (contours, hierarchy) in cv2's
+    shapes.  Every Contour carries `points` (int32 [n,1,2], the array cv2 returns for that border), `is_hole` and the
+    Green's-theorem sums, so contour_centroid / contour_area apply to it; hierarchy is int32 [1,N,4] (next, prev,
+    first_child, parent), or None when there is no border, as cv2 returns it.
+    mode: "external", "list", "ccomp" or "tree"; method: "none" or "simple".  The borders are the ones cv2 finds, each
+    with cv2's vertex list, ordered outer borders first (raster order of their first pixel), then hole borders (raster
+    order of the hole); cv2 orders them its own way.  "external" is outer_contours(points=True) with cv2's flat
+    hierarchy.  max_contours / max_points are first guesses: when a frame needs more, the call is repeated with room for
+    everything it reported."""
+    from .runtime import CONTOUR_DTYPE
+    if mode == "external":
+        if method != "simple":
+            raise ValueError("mode 'external' is served with CHAIN_APPROX_SIMPLE only")
+        ctx = ctx_for(mat)
+        dev = to_device(ctx, mat)
+        h, w = mat.shape[-2], mat.shape[-1]
+        _, nb, _, _ = ctx.outer_contours(dev, max_contours=max_contours)
+        max_contours = max(max_contours, int(ctx.download(nb)[0]))
+        max_points = max(max_points or 0, 4 * (h + w) + h * w // 4)
+        out = outer_contours(dev, max_contours=max_contours, points=True, max_points=max_points)
+        for c in out:
+            c["is_hole"] = False
+        n = len(out)
+        hier = np.array([[[i + 1 if i + 1 < n else -1, i - 1, -1, -1] for i in range(n)]], np.int32).reshape(1, n, 4)
+        return out, (hier if n else None)
+    ctx = ctx_for(mat)
+    h, w = mat.shape[-2], mat.shape[-1]
+    dev = to_device(ctx, mat)
+    if max_points is None:
+        max_points = 4 * (h + w) + h * w // 4
+    # at most three calls: the vertex count covers the written records only, so it is complete once the records fit
+    for _ in range(3):
+        table, hier, nc, pts, npts = ctx.find_contours(dev, mode, method, max_contours=max_contours,
+                                                       max_points=max_points)
+        n_outer, n_holes = (int(v) for v in ctx.download(nc)[0])
+        needed = int(ctx.download(npts)[0])
+        if n_outer + n_holes <= max_contours and needed <= max_points:
+            break
+        max_contours, max_points = max(max_contours, n_outer + n_holes), max(max_points, needed)
+    n = n_outer + n_holes
+    raw = ctx.download(table)[0, :n].copy().view(CONTOUR_DTYPE).reshape(-1)
+    host = ctx.download(pts)[0, :needed]
+    none = method in ("none", ctx.CHAIN["none"])
+    out = []
+    for i in range(n):
+        c = Contour({k: int(raw[i][k]) for k in CONTOUR_DTYPE.names})
+        c["is_hole"] = i >= n_outer
+        off, cnt = c["point_offset"], c["n_points"] if none else c["n_simple"]
+        c["points"] = host[off:off + cnt].reshape(-1, 1, 2).copy()
+        out.append(c)
+    return out, (ctx.download(hier)[:1, :n].copy() if n else None)
 
 
 def _contour_moments(c):

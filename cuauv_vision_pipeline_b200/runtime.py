@@ -323,6 +323,29 @@ class Context:
                                     ffi.cast("int32_t *", npts.data_ptr()) if max_points else ffi.NULL))
         return table, nb, points, npts
 
+    RETR = {"list": lib.BV_RETR_LIST, "ccomp": lib.BV_RETR_CCOMP, "tree": lib.BV_RETR_TREE}
+    CHAIN = {"none": lib.BV_CHAIN_APPROX_NONE, "simple": lib.BV_CHAIN_APPROX_SIMPLE}
+
+    def find_contours(self, mask, mode="tree", method="simple", max_contours=4096, max_points=0):
+        """cv2.findContours(mask, RETR_LIST / CCOMP / TREE, CHAIN_APPROX_NONE / SIMPLE) of a device mask [H,W] or
+        [B,H,W] -> (contour table as uint8 [B,max,72]: outer borders then hole borders, hierarchy int32
+        [B,max,4], counts int32 [B,2] = (outer, holes), points int32 [B,max_points,2] or None, points needed [B]
+        or None).  `mode` / `method` take the names or the BV_* values."""
+        mode = self.RETR[mode] if isinstance(mode, str) else int(mode)
+        method = self.CHAIN[method] if isinstance(method, str) else int(method)
+        b, h, w, _ = self._bhw(mask, channels=1)
+        table = self.empty((b, max_contours, CONTOUR_DTYPE.itemsize), torch.uint8)
+        hier = self.empty((b, max_contours, 4), torch.int32)
+        nc = self.empty((b, 2), torch.int32)
+        points = self.empty((b, max_points, 2), torch.int32) if max_points else None
+        npts = self.empty((b,), torch.int32) if max_points else None
+        check(lib.bv_find_contours(self.handle, _u8ptr(mask), b, h, w, mode, method,
+                                   ffi.cast("bv_contour *", table.data_ptr()), ffi.cast("int32_t *", hier.data_ptr()),
+                                   max_contours, ffi.cast("int32_t *", nc.data_ptr()),
+                                   ffi.cast("int32_t *", points.data_ptr()) if max_points else ffi.NULL, max_points,
+                                   ffi.cast("int32_t *", npts.data_ptr()) if max_points else ffi.NULL))
+        return table, hier, nc, points, npts
+
     def min_area_rects(self, table, nb, points):
         """cv2.minAreaRect of every external contour of `outer_contours(..., max_points > 0)`: structured numpy
         array [B, max_contours] with fields cx, cy, width, height, angle, valid."""

@@ -232,10 +232,13 @@ typedef struct bv_contour {
     int64_t a00, a10, a01;
     int32_t x0, y0, x1, y1;   /* bounding box of the border pixels (inclusive)                    */
     int32_t start_x, start_y; /* first border pixel = the component's first pixel in raster order */
+                              /* (hole border, bv_find_contours: the pixel left of the hole's)    */
     int32_t n_points;         /* border pixels visited (length of the CHAIN_APPROX_NONE contour)  */
     int32_t n_simple;         /* vertices kept by CHAIN_APPROX_SIMPLE (utils/feature.py:20)       */
-    int32_t label;            /* the component's label in bv_label's numbering                    */
+    int32_t label;            /* the component's label in bv_label's numbering (hole border: the  */
+                              /* label of the component around the hole)                          */
     int32_t external;         /* 1: reported by RETR_EXTERNAL; 0: lies inside another blob's hole */
+                              /* or is a hole border                                              */
     int32_t point_offset;     /* index of its first vertex in the frame's point list, -1 if the   */
                               /* list was not requested or is full                                */
     int32_t reserved;
@@ -251,6 +254,39 @@ typedef struct bv_contour {
 int bv_outer_contours(bv_ctx *ctx, const uint8_t *mask_dev, int batch, int height, int width,
                       bv_contour *contours_dev, int max_contours, int32_t *n_contours_dev, int32_t *points_dev,
                       int max_points, int32_t *n_points_dev);
+
+/* Every border of cv2.findContours(mask, mode, method) with its hierarchy (utils/feature.py:25-40
+ * all_contours; vision_common.py Hierarchy / fill_ratio).  Values are cv2's. */
+typedef enum bv_retr_mode {
+    BV_RETR_LIST = 1,  /* no hierarchy: every parent and child is -1                                */
+    BV_RETR_CCOMP = 2, /* outer borders at the top level, each hole a child of its component's border */
+    BV_RETR_TREE = 3   /* the full nesting                                                           */
+} bv_retr_mode;
+typedef enum bv_chain_approx {
+    BV_CHAIN_APPROX_NONE = 1,  /* every border pixel                                               */
+    BV_CHAIN_APPROX_SIMPLE = 2 /* the pixels where the chain turns (cyclically, so the start of a  */
+                               /* hole border is dropped when the chain runs straight through it)  */
+} bv_chain_approx;
+/* The same set of borders as cv2 (one outer border per 8-connected component, one hole border per
+ * 4-connected background region that does not touch the image edge), in this order, per frame:
+ *   records 0 .. n_outer-1: the outer borders, in bv_label's label order, equal to the records
+ *     bv_outer_contours writes;
+ *   records n_outer .. n_outer+n_holes-1: the hole borders, in raster order of the hole's first
+ *     pixel; start_x/start_y = the pixel left of it, label = the enclosing component's label,
+ *     external = 0.
+ * cv2 lists the same borders in an order of its own; each border's vertex list is identical.
+ * contours_dev: bv_contour[batch * max_contours].  hierarchy_dev (optional, 16-byte aligned):
+ * int32[batch][max_contours][4] = cv2's (next, prev, first_child, parent) over this record order;
+ * siblings are linked in increasing record order and first_child is the smallest child.
+ * n_contours_dev (optional): int32[batch][2] = (n_outer, n_holes), which may exceed max_contours:
+ * records past max_contours are not written, and hierarchy links then reach only written records.
+ * points_dev (optional): int32[batch][max_points][2] receiving the vertices (x, y) of every record
+ * in cv2's order, record after record; n_points_dev (optional): int32[batch] vertices the written
+ * records need per frame (may exceed max_points: records that do not fit get point_offset = -1).
+ * mode = BV_RETR_EXTERNAL (cv2's 0) is bv_outer_contours. */
+int bv_find_contours(bv_ctx *ctx, const uint8_t *mask_dev, int batch, int height, int width, int mode, int method,
+                     bv_contour *contours_dev, int32_t *hierarchy_dev, int max_contours, int32_t *n_contours_dev,
+                     int32_t *points_dev, int max_points, int32_t *n_points_dev);
 
 /* cv2.minAreaRect of every external contour (modules/bins.py:60-69; utils/feature.py:301-312), from
  * the vertex lists bv_outer_contours wrote (same contours_dev / n_contours_dev / points_dev /
