@@ -18,6 +18,7 @@
 //   (float32 products scaled by 2^15, rounded, largest/smallest entry adjusted so that they sum
 //   to 2^15); result (sum + 2^14) >> 15.  Taps outside the image replicate the edge
 //   (BORDER_REPLICATE) or take the border value (BORDER_CONSTANT).
+#include <limits.h>
 #include <math.h>
 
 #include "common.cuh"
@@ -309,11 +310,19 @@ struct WarpParams {
     int border_value[4];
 };
 
+// cvRound / saturate_cast<int> of OpenCV on x86-64 (cvtsd2si, cvtss2si): round half to even; NaN, +-inf and every value
+// whose rounded result lies outside int32 give INT_MIN ("integer indefinite"), on either side.
 __device__ __forceinline__ int sat_round_int(double v) {
-    if (v >= 2147483647.0) return 2147483647;
-    if (v <= -2147483648.0) return (int)0x80000000;
-    return __double2int_rn(v);  // cvRound: nearest even
+    const double r = rint(v);
+    return r >= -2147483648.0 && r <= 2147483647.0 ? (int)r : INT_MIN;
 }
+
+__device__ __forceinline__ int sat_round_int(float v) {
+    const float r = rintf(v);
+    return r >= -2147483648.f && r < 2147483648.f ? (int)r : INT_MIN;
+}
+
+__device__ __forceinline__ short sat_short(int v) { return (short)(v < -32768 ? -32768 : (v > 32767 ? 32767 : v)); }
 
 // The fixed-point coordinate terms depend on the column (adelta, bdelta) or on the row (X0, Y0) only: OpenCV
 // tabulates them per call, and so does this kernel's small prologue launch (coords = [adelta | bdelta | X0 | Y0]).
@@ -406,15 +415,14 @@ __global__ void __launch_bounds__(256) warp_affine_kernel(const uint8_t *__restr
     const int adelta = __ldg(coords + x), bdelta = __ldg(coords + dst_w + x);
     const int X0 = __ldg(coords + 2 * dst_w + y), Y0 = __ldg(coords + 2 * dst_w + dst_h + y);
     const int X = (X0 + adelta) >> (AB_BITS - INTER_BITS), Y = (Y0 + bdelta) >> (AB_BITS - INTER_BITS);
-    int sx = X >> INTER_BITS, sy = Y >> INTER_BITS;
-    sx = sx < -32768 ? -32768 : (sx > 32767 ? 32767 : sx);  // saturate_cast<short>
-    sy = sy < -32768 ? -32768 : (sy > 32767 ? 32767 : sy);
+    const int sx = sat_short(X >> INTER_BITS), sy = sat_short(Y >> INTER_BITS);  // saturate_cast<short>
     bilinear_sample<CN>(f, frame_bytes, words_ok, height, width, sx, sy, (Y & (TAB - 1)) * TAB + (X & (TAB - 1)), tab, wp, o);
 }
 
 // cv2.remap(INTER_LINEAR) on uint8.  FIXED: map1 = int16 (x, y) pairs, map2 = uint16 fy * 32 + fx (CV_16SC2 + CV_16UC1).
 // Otherwise map1 / map2 are float32 x / y planes, converted the way RemapInvoker converts them block by block:
-// cvRound(x * 32) in float32, integer part saturated to short, the two 5-bit fractions.
+// cvRound(x * 32) in float32 (NaN, +-inf and |x * 32| >= 2^31 give INT_MIN, so such a tap lands on the left / top border),
+// integer part saturated to short, the two 5-bit fractions.
 template <int CN, bool FIXED>
 __global__ void __launch_bounds__(256) remap_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, int height, int width,
                                                     int dst_h, int dst_w, const void *__restrict__ map1, const void *__restrict__ map2,
@@ -433,12 +441,10 @@ __global__ void __launch_bounds__(256) remap_kernel(const uint8_t *__restrict__ 
         sy = xy.y;
         frac = __ldg(static_cast<const unsigned short *>(map2) + i) & 1023;
     } else {
-        const int X = __float2int_rn(__fmul_rn(__ldg(static_cast<const float *>(map1) + i), 32.f));
-        const int Y = __float2int_rn(__fmul_rn(__ldg(static_cast<const float *>(map2) + i), 32.f));
-        sx = X >> 5;
-        sy = Y >> 5;
-        sx = sx < -32768 ? -32768 : (sx > 32767 ? 32767 : sx);  // saturate_cast<short>
-        sy = sy < -32768 ? -32768 : (sy > 32767 ? 32767 : sy);
+        const int X = sat_round_int(__fmul_rn(__ldg(static_cast<const float *>(map1) + i), 32.f));
+        const int Y = sat_round_int(__fmul_rn(__ldg(static_cast<const float *>(map2) + i), 32.f));
+        sx = sat_short(X >> 5);  // saturate_cast<short>
+        sy = sat_short(Y >> 5);
         frac = (Y & 31) * 32 + (X & 31);
     }
     bilinear_sample<CN>(f, frame_bytes, words_ok, height, width, sx, sy, frac, tab, wp, o);
@@ -485,7 +491,7 @@ __global__ void __launch_bounds__(256) undistort_maps_kernel(UndistortParams p, 
     }
     if (xy) {
         const int iu = sat_round_int(us * 32.0), iv = sat_round_int(vs * 32.0);  // saturate_cast<int>(u * INTER_TAB_SIZE)
-        xy[o] = make_short2((short)(iu >> 5), (short)(iv >> 5));
+        xy[o] = make_short2(sat_short(iu >> 5), sat_short(iv >> 5));  // saturate_cast<short>
         frac[o] = (unsigned short)((iv & 31) * 32 + (iu & 31));
     }
 }
@@ -604,14 +610,10 @@ extern "C" int bv_gaussian_blur(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *ds
         BV_REQUIRE(height <= 65535, "image too tall");
         BV_TRY(ensure_scratch(ctx, SCR_MORPH_TMP, (size_t)batch * height * width * channels * sizeof(uint16_t)));
         uint16_t *hz = (uint16_t *)ctx->scratch[SCR_MORPH_TMP];
+        // only 3-channel images get here: the largest 1-channel tile (201 x 201 taps) needs 90 944 bytes
         dim3 g((width + 255) / 256, height, batch);
-        if (channels == 3) {
-            BV_LAUNCH(ctx, blur_rows16_kernel<3>, g, 256, 0, src_dev, hz, height, width, taps);
-            BV_LAUNCH(ctx, blur_cols16_kernel<3>, g, 256, 0, hz, dst_dev, height, width, taps);
-        } else {
-            BV_LAUNCH(ctx, blur_rows16_kernel<1>, g, 256, 0, src_dev, hz, height, width, taps);
-            BV_LAUNCH(ctx, blur_cols16_kernel<1>, g, 256, 0, hz, dst_dev, height, width, taps);
-        }
+        BV_LAUNCH(ctx, blur_rows16_kernel<3>, g, 256, 0, src_dev, hz, height, width, taps);
+        BV_LAUNCH(ctx, blur_cols16_kernel<3>, g, 256, 0, hz, dst_dev, height, width, taps);
         return BV_OK;
     }
     dim3 grid((width + kBlurTileW - 1) / kBlurTileW, (height + kBlurTileH - 1) / kBlurTileH, batch);

@@ -141,6 +141,13 @@ class Context:
             return t.shape[0], t.shape[1], t.shape[2], t.shape[3]
         raise BVError(-1, "unsupported tensor rank")
 
+    def _src(self, t):
+        """A source image of the filter, morphology and noise steps: a contiguous uint8 tensor on this context's device
+        (the kernels read it as packed bytes)."""
+        if t.dtype != torch.uint8 or t.device != self.device or not t.is_contiguous():
+            raise BVError(-1, "expected a contiguous uint8 tensor on %s" % self.device)
+        return t
+
     def cvt_color(self, src, code, split=False):
         code_i = CVT[code] if isinstance(code, str) else int(code)
         if code_i != lib.BV_GRAY2BGR:
@@ -259,6 +266,7 @@ class Context:
         return np.float32(out[0])
 
     def morph(self, src, op, kernel, iterations=1):
+        self._src(src)
         kernel = np.ascontiguousarray(np.asarray(kernel) != 0, dtype=np.uint8)
         kh, kw = kernel.shape
         if src.dim() == 2:
@@ -384,7 +392,7 @@ class Context:
 
     def gaussian_blur(self, src, ksize, sigma_x=0.0, sigma_y=0.0):
         """cv2.GaussianBlur(src, ksize=(kw, kh), sigma_x, sigma_y) on uint8 (BORDER_REFLECT_101)."""
-        b, h, w, c = self._bhwc(src)
+        b, h, w, c = self._bhwc(self._src(src))
         dst = self.empty(tuple(src.shape))
         check(lib.bv_gaussian_blur(self.handle, _u8ptr(src), _u8ptr(dst), b, h, w, c, int(ksize[0]), int(ksize[1]),
                                    float(sigma_x), float(sigma_y)))
@@ -392,7 +400,7 @@ class Context:
 
     def warp_affine(self, src, matrix, dsize=None, border="constant", border_value=(0, 0, 0)):
         """cv2.warpAffine(src, matrix, dsize, flags=INTER_LINEAR, borderMode=..., borderValue=...) on uint8."""
-        b, h, w, c = self._bhwc(src)
+        b, h, w, c = self._bhwc(self._src(src))
         dw, dh = (w, h) if dsize is None else (int(dsize[0]), int(dsize[1]))
         m = np.ascontiguousarray(np.asarray(matrix, dtype=np.float64).reshape(6))
         bv_ = np.ascontiguousarray(np.asarray(list(border_value)[:c] + [0] * max(0, c - len(border_value)), dtype=np.uint8))
@@ -405,15 +413,15 @@ class Context:
     def remap(self, src, map1, map2, border="constant", border_value=(0, 0, 0)):
         """cv2.remap(src, map1, map2, INTER_LINEAR, borderMode, borderValue) on uint8.  Device maps: two float32 [H,W]
         planes (x, y) or int16 [H,W,2] + uint16 [H,W] (fixed point)."""
-        b, h, w, c = self._bhwc(src)
+        b, h, w, c = self._bhwc(self._src(src))
         fixed = map1.dtype == torch.int16
         if fixed:
             if map1.dim() != 3 or map1.shape[2] != 2 or map2.dtype not in (torch.uint16, torch.int16) or tuple(map2.shape) != tuple(map1.shape[:2]):
                 raise BVError(-1, "fixed-point maps are int16 [H,W,2] + uint16 [H,W]")
         elif map1.dtype != torch.float32 or map2.dtype != torch.float32 or map1.dim() != 2 or tuple(map1.shape) != tuple(map2.shape):
             raise BVError(-1, "float maps are two float32 [H,W] planes")
-        if not (map1.is_cuda and map2.is_cuda and map1.is_contiguous() and map2.is_contiguous()):
-            raise BVError(-1, "maps must be contiguous CUDA tensors")
+        if not (map1.device == self.device == map2.device and map1.is_contiguous() and map2.is_contiguous()):
+            raise BVError(-1, "maps must be contiguous tensors on %s" % self.device)
         dh, dw = int(map1.shape[0]), int(map1.shape[1])
         bv_ = np.ascontiguousarray(np.asarray(list(border_value)[:c] + [0] * max(0, c - len(border_value)), dtype=np.uint8))
         shape = (dh, dw) if src.dim() == 2 else ((dh, dw, c) if src.dim() == 3 else (b, dh, dw, c))
@@ -445,7 +453,7 @@ class Context:
 
     def lab_shift_local_mean(self, lab, ksize):
         """a, b of a uint8 LAB image minus (their ksize x ksize box mean - 128), numpy-cast to uint8 (white_balance_bgr_blur)."""
-        b, h, w, c = self._bhwc(lab)
+        b, h, w, c = self._bhwc(self._src(lab))
         if c != 3:
             raise BVError(-1, "lab_shift_local_mean needs a 3-channel image")
         dst = self.empty(tuple(lab.shape))
@@ -456,6 +464,7 @@ class Context:
         """clip(src + randn(*src.shape) * sigma, 0, 255).astype(uint8) with the values numpy's legacy generator would
         draw: numpy's global one (as modules/preprocessor.py:115-119 uses) unless a RandomState is given.  The
         generator is advanced exactly as numpy.random.randn would advance it."""
+        self._src(src)
         rs = np.random if random_state is None else random_state
         name, key, pos, has_gauss, cached = rs.get_state()
         if name != "MT19937":

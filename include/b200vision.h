@@ -331,8 +331,10 @@ int bv_warp_affine(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int ba
  * definition or call site, so parity is pinned to the cv2 calls such a definition makes).
  * bv_remap == cv2.remap(src, map1, map2, INTER_LINEAR, borderMode, borderValue) on uint8; the maps live on the device and
  * serve every frame of the batch.  BV_MAP_F32: map1 / map2 are float32 x / y planes (CV_32FC1); BV_MAP_FIXED: map1 is
- * int16 (x, y) pairs, map2 uint16 (fy * 32 + fx) (CV_16SC2 + CV_16UC1, what cv2.convertMaps and cv2.undistort use).
- * Bit-exact in both formats. */
+ * int16 (x, y) pairs, map2 uint16 (fy * 32 + fx, read & 1023 as cv2 does) (CV_16SC2 + CV_16UC1, what cv2.convertMaps and
+ * cv2.undistort use).  A float map value becomes cvRound(x * 32) as OpenCV computes it on x86-64: round half to even, and
+ * INT_MIN for NaN, +-inf and |x * 32| >= 2^31 (such a tap lands on the left / top border, whichever its sign); the
+ * integer part is then saturated to int16.  Bit-exact in both formats.  src_dev != dst_dev. */
 typedef enum bv_map_format { BV_MAP_F32 = 0, BV_MAP_FIXED = 1 } bv_map_format;
 int bv_remap(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width, int channels,
              int dst_height, int dst_width, const void *map1_dev, const void *map2_dev, int map_format, int border_mode,
@@ -342,7 +344,10 @@ int bv_remap(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, i
  * straight from the float64 coordinates; either pair may be NULL.  camera_matrix_host: 3x3 row-major; dist_coeffs_host:
  * n_dist = 0, 4, 5 or 8 values k1 k2 p1 p2 [k3 [k4 k5 k6]]; inv_new_camera_rot_host: inverse of
  * (new_camera_matrix x R), 3x3 row-major.  float64 arithmetic in OpenCV's order: identical maps on the reference's
- * camera files (lib/configs/<n>_camera_matrix_params.yaml); in general to the last float32 bit. */
+ * camera files (lib/configs/<n>_camera_matrix_params.yaml); in general to the last float32 bit.  Fixed-point pair:
+ * saturate_cast<int>(u * 32) (INT_MIN for NaN and values beyond int32, as cvRound on x86-64), integer part saturated to
+ * int16 as cv2's vector code does (cv2's scalar code for the last width mod (2 x float64 lanes) columns of a row
+ * truncates instead; the two agree wherever a ray stays within int16). */
 int bv_undistort_maps(bv_ctx *ctx, const double *camera_matrix_host, const double *dist_coeffs_host, int n_dist,
                       const double *inv_new_camera_rot_host, int width, int height, float *mapx_dev, float *mapy_dev,
                       int16_t *map_xy_dev, uint16_t *map_frac_dev);

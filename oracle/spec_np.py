@@ -294,6 +294,25 @@ def _bilinear_tab():
     return tab
 
 
+INT_MIN = -2 ** 31
+
+
+def cv_round(v):
+    """cvRound / saturate_cast<int> of a float32 or float64 value as OpenCV computes it on x86-64 (cvtss2si, cvtsd2si):
+    round half to even; NaN, +-inf and every value whose rounded result lies outside int32 give INT_MIN, on either side
+    ("integer indefinite").  So a huge positive coordinate lands on the left / top edge, not the right / bottom one."""
+    v = np.asarray(v)
+    with np.errstate(invalid="ignore"):
+        r = np.rint(v).astype(np.float64)              # exact: rint of a float32 is a float32 integer
+        ok = (r >= -2.0 ** 31) & (r <= 2.0 ** 31 - 1)
+    return np.where(ok, np.where(ok, r, 0).astype(np.int64), np.int64(INT_MIN))
+
+
+def wrap_int32(v):
+    """int32 arithmetic of C on two's complement: the int64 value reduced mod 2^32."""
+    return ((np.asarray(v, np.int64) + 2 ** 31) & 0xFFFFFFFF) - 2 ** 31
+
+
 def rotation_matrix_2d(center, angle, scale):
     a = angle * (np.pi / 180)          # cv2: angle *= CV_PI/180
     alpha, beta = np.cos(a) * scale, np.sin(a) * scale
@@ -308,26 +327,28 @@ def warp_affine_8u(img, matrix, dsize=None, border="constant", border_value=0):
     h, w = img.shape[:2]
     dw, dh = (w, h) if dsize is None else dsize
     m = np.asarray(matrix, np.float64).reshape(6).copy()
-    d = m[0] * m[4] - m[1] * m[3]
-    d = 1.0 / d if d != 0 else 0.0
-    a11, a22 = m[4] * d, m[0] * d
-    m[0], m[1], m[3], m[4] = a11, m[1] * -d, m[3] * -d, a22
-    b1 = -m[0] * m[2] - m[1] * m[5]
-    b2 = -m[3] * m[2] - m[4] * m[5]
+    with np.errstate(invalid="ignore", divide="ignore"):      # NaN / inf entries propagate as in cv2
+        d = m[0] * m[4] - m[1] * m[3]
+        d = 1.0 / d if d != 0 else 0.0
+        a11, a22 = m[4] * d, m[0] * d
+        m[0], m[1], m[3], m[4] = a11, m[1] * -d, m[3] * -d, a22
+        b1 = -m[0] * m[2] - m[1] * m[5]
+        b2 = -m[3] * m[2] - m[4] * m[5]
     m[2], m[5] = b1, b2
     tab = _bilinear_tab()
 
-    def rnd(v):
-        return np.clip(np.rint(v), -2.0 ** 31, 2.0 ** 31 - 1).astype(np.int64)
+    rnd = cv_round                                     # saturate_cast<int>(double)
     xs = np.arange(dw, dtype=np.float64)
-    adelta, bdelta = rnd(m[0] * xs * 1024.0), rnd(m[3] * xs * 1024.0)
+    with np.errstate(invalid="ignore"):                # NaN / inf matrix entries
+        adelta, bdelta = rnd(m[0] * xs * 1024.0), rnd(m[3] * xs * 1024.0)
     out = np.zeros((dh, dw, img.shape[2]), np.uint8)
     src = img.astype(np.int64)
     bval = np.broadcast_to(np.asarray(border_value, np.int64), (img.shape[2],))
     for y in range(dh):
-        x0 = int(rnd(np.float64((m[1] * y + m[2]) * 1024.0))) + 16
-        y0 = int(rnd(np.float64((m[4] * y + m[5]) * 1024.0))) + 16
-        X, Y = (x0 + adelta) >> 5, (y0 + bdelta) >> 5
+        with np.errstate(invalid="ignore"):
+            x0 = int(rnd(np.float64((m[1] * y + m[2]) * 1024.0))) + 16
+            y0 = int(rnd(np.float64((m[4] * y + m[5]) * 1024.0))) + 16
+        X, Y = wrap_int32(x0 + adelta) >> 5, wrap_int32(y0 + bdelta) >> 5      # int additions wrap
         sx, sy = np.clip(X >> 5, -32768, 32767), np.clip(Y >> 5, -32768, 32767)
         wt = tab[(Y & 31) * 32 + (X & 31)]                               # [dw, 4]
         acc = np.zeros((dw, img.shape[2]), np.int64)
@@ -349,9 +370,11 @@ def warp_affine_8u(img, matrix, dsize=None, border="constant", border_value=0):
 # ---------------------------------------------------------------------------------------------
 def fixed_point_maps(mapx, mapy):
     """float32 maps -> (int16 xy [H,W,2], uint16 fractional index [H,W]) as RemapInvoker converts them per block:
-    cvRound(float32(x) * 32), integer part saturated to short, 5-bit fractions combined into fy*32 + fx."""
-    sx = np.rint(np.asarray(mapx, np.float32) * np.float32(32)).astype(np.int64)
-    sy = np.rint(np.asarray(mapy, np.float32) * np.float32(32)).astype(np.int64)
+    cvRound(float32(x) * 32) (INT_MIN for NaN, +-inf and |x * 32| >= 2^31, see cv_round), integer part saturated to
+    short, 5-bit fractions combined into fy*32 + fx."""
+    with np.errstate(invalid="ignore", over="ignore"):
+        sx = cv_round(np.asarray(mapx, np.float32) * np.float32(32))
+        sy = cv_round(np.asarray(mapy, np.float32) * np.float32(32))
     xy = np.stack([np.clip(sx >> 5, -32768, 32767), np.clip(sy >> 5, -32768, 32767)], axis=-1).astype(np.int16)
     return xy, ((sy & 31) * 32 + (sx & 31)).astype(np.uint16)
 
@@ -404,8 +427,9 @@ def init_undistort_rectify_map(camera_matrix, dist_coeffs, new_camera_matrix, si
     xd = x * kr + p1 * _2xy + p2 * (r2 + 2 * x2)
     yd = y * kr + p1 * (r2 + 2 * y2) + p2 * _2xy
     us, vs = fx * xd + cx, fy * yd + cy
-    if fixed:   # the CV_16SC2 + CV_16UC1 pair, rounded straight from the doubles (what cv2.undistort builds)
-        iu = np.clip(np.rint(us * 32), -2.0 ** 31, 2.0 ** 31 - 1).astype(np.int64)
-        iv = np.clip(np.rint(vs * 32), -2.0 ** 31, 2.0 ** 31 - 1).astype(np.int64)
-        return np.stack([iu >> 5, iv >> 5], axis=-1).astype(np.int16), ((iv & 31) * 32 + (iu & 31)).astype(np.uint16)
+    if fixed:   # the CV_16SC2 + CV_16UC1 pair, rounded straight from the doubles (what cv2.undistort builds):
+        # saturate_cast<int>(u * 32) (see cv_round), then saturate_cast<short> of the integer part
+        iu, iv = cv_round(us * 32), cv_round(vs * 32)
+        xy = np.stack([np.clip(iu >> 5, -32768, 32767), np.clip(iv >> 5, -32768, 32767)], axis=-1).astype(np.int16)
+        return xy, ((iv & 31) * 32 + (iu & 31)).astype(np.uint16)
     return us.astype(np.float32), vs.astype(np.float32)
