@@ -69,7 +69,8 @@ def outer_contours(mat, max_contours=4096, points=False, max_points=None, rects=
     return out
 
 
-def find_contours(mat, mode="tree", method="simple", max_contours=4096, max_points=None):
+def find_contours(mat, mode="tree", method="simple", max_contours=4096, max_points=None, shapes=False, approx_epsilon=0.0,
+                  approx_relative=0.0):
     """cv2.findContours(mat, RETR_<mode>, CHAIN_APPROX_<method>) on the GPU for one mask: (contours, hierarchy) in cv2's
     shapes.  Every Contour carries `points` (int32 [n,1,2], the array cv2 returns for that border), `is_hole` and the
     Green's-theorem sums, so contour_centroid / contour_area apply to it; hierarchy is int32 [1,N,4] (next, prev,
@@ -78,7 +79,12 @@ def find_contours(mat, mode="tree", method="simple", max_contours=4096, max_poin
     with cv2's vertex list, ordered outer borders first (raster order of their first pixel), then hole borders (raster
     order of the hole); cv2 orders them its own way.  "external" is outer_contours(points=True) with cv2's flat
     hierarchy.  max_contours / max_points are first guesses: when a frame needs more, the call is repeated with room for
-    everything it reported."""
+    everything it reported.
+    With `shapes=True` every Contour also carries its shape descriptors, computed on the device (bv_contour_shapes):
+    `arc_length` (cv2.arcLength(points, True)), `hull` (cv2.convexHull(points), int32 [k,1,2]), `approx`
+    (cv2.approxPolyDP(points, approx_epsilon + approx_relative * arc_length, True), int32 [k,1,2]), `approx_convex`
+    (cv2.isContourConvex(approx)), `min_enclosing_circle` ((cx, cy), r) and `min_area_rect` ((cx, cy), (w, h), angle),
+    hole borders included."""
     from .runtime import CONTOUR_DTYPE
     if mode == "external":
         if method != "simple":
@@ -89,7 +95,10 @@ def find_contours(mat, mode="tree", method="simple", max_contours=4096, max_poin
         _, nb, _, _ = ctx.outer_contours(dev, max_contours=max_contours)
         max_contours = max(max_contours, int(ctx.download(nb)[0]))
         max_points = max(max_points or 0, 4 * (h + w) + h * w // 4)
-        out = outer_contours(dev, max_contours=max_contours, points=True, max_points=max_points)
+        if shapes:
+            out = _outer_with_shapes(ctx, dev, max_contours, max_points, approx_epsilon, approx_relative)
+        else:
+            out = outer_contours(dev, max_contours=max_contours, points=True, max_points=max_points)
         for c in out:
             c["is_hole"] = False
         n = len(out)
@@ -120,7 +129,49 @@ def find_contours(mat, mode="tree", method="simple", max_contours=4096, max_poin
         off, cnt = c["point_offset"], c["n_points"] if none else c["n_simple"]
         c["points"] = host[off:off + cnt].reshape(-1, 1, 2).copy()
         out.append(c)
+    if shapes:
+        _attach_shapes(ctx, out, range(n), table, nc, pts, method, approx_epsilon, approx_relative)
     return out, (ctx.download(hier)[:1, :n].copy() if n else None)
+
+
+def _outer_with_shapes(ctx, dev, max_contours, max_points, approx_epsilon, approx_relative):
+    """The external borders with their vertices and shape descriptors, all from one bv_outer_contours table that is
+    grown until every border and every vertex fits."""
+    from .runtime import CONTOUR_DTYPE
+    for _ in range(3):
+        table, nb, pts, npts = ctx.outer_contours(dev, max_contours=max_contours, max_points=max_points)
+        n, needed = int(ctx.download(nb)[0]), int(ctx.download(npts)[0])
+        if n <= max_contours and needed <= max_points:
+            break
+        max_contours, max_points = max(max_contours, n), max(max_points, needed)
+    raw = ctx.download(table)[0, :n].copy().view(CONTOUR_DTYPE).reshape(-1)
+    keep = [i for i, row in enumerate(raw) if row["external"]]
+    out = [Contour({k: int(raw[i][k]) for k in CONTOUR_DTYPE.names}) for i in keep]
+    host = ctx.download(pts)[0, :needed]
+    for c in out:
+        off = c["point_offset"]
+        c["points"] = host[off:off + c["n_simple"]].reshape(-1, 1, 2).copy()
+    _attach_shapes(ctx, out, keep, table, nb, pts, "simple", approx_epsilon, approx_relative)
+    return out
+
+
+def _attach_shapes(ctx, out, records, table, counts, pts, method, approx_epsilon, approx_relative):
+    """Adds the bv_contour_shapes descriptors of record records[k] to out[k]."""
+    from .runtime import SHAPE_DTYPE
+    shapes, hull, approx = ctx.contour_shapes(table, counts, pts, method, approx_epsilon, approx_relative)
+    sh = ctx.download(shapes)[0].copy().view(SHAPE_DTYPE).reshape(-1)
+    hull, approx = ctx.download(hull)[0], ctx.download(approx)[0]
+    for c, i in zip(out, records):
+        s, off = sh[i], c["point_offset"]
+        if not s["valid"]:
+            raise RuntimeError("contour record %d has no shape descriptors" % i)
+        r = s["rect"]
+        c["arc_length"] = float(s["arc_length"])
+        c["hull"] = hull[off:off + int(s["n_hull"])].reshape(-1, 1, 2).copy()
+        c["approx"] = approx[off:off + int(s["n_approx"])].reshape(-1, 1, 2).copy()
+        c["approx_convex"] = bool(s["approx_convex"])
+        c["min_enclosing_circle"] = ((float(s["circle_cx"]), float(s["circle_cy"])), float(s["circle_r"]))
+        c["min_area_rect"] = ((float(r["cx"]), float(r["cy"])), (float(r["width"]), float(r["height"])), float(r["angle"]))
 
 
 def _contour_moments(c):

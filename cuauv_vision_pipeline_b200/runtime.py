@@ -31,6 +31,10 @@ CONTOUR_DTYPE = np.dtype([(k, "<i8") for k in ("a00", "a10", "a01")] +
 assert CONTOUR_DTYPE.itemsize == ffi.sizeof("bv_contour")
 RRECT_DTYPE = np.dtype([(k, "<f4") for k in ("cx", "cy", "width", "height", "angle")] + [("valid", "<i4")])
 assert RRECT_DTYPE.itemsize == ffi.sizeof("bv_rrect")
+SHAPE_DTYPE = np.dtype([("arc_length", "<f8")] + [(k, "<f4") for k in ("circle_cx", "circle_cy", "circle_r")] +
+                       [("rect", RRECT_DTYPE)] + [(k, "<i4") for k in ("n_hull", "n_approx", "approx_convex", "valid",
+                                                                      "reserved")])
+assert SHAPE_DTYPE.itemsize == ffi.sizeof("bv_shape")
 
 
 def _u8ptr(t):
@@ -364,6 +368,27 @@ class Context:
                                     ffi.cast("int32_t *", points.data_ptr()), b, max_contours, max_points,
                                     ffi.cast("bv_rrect *", rects.data_ptr())))
         return self.download(rects).view(RRECT_DTYPE).reshape(b, max_contours)
+
+    def contour_shapes(self, table, counts, points, method, approx_epsilon=0.0, approx_relative=0.0, hull=True,
+                       approx=True):
+        """Shape descriptors of every record of a contour table (bv_contour_shapes): `table`, `counts` and `points` as
+        find_contours (counts [B,2]) or outer_contours (counts [B], SIMPLE) returned them.  Returns (shapes as uint8
+        [B,max_contours,SHAPE_DTYPE.itemsize], hull int32 [B,max_points,2] or None, approx int32 [B,max_points,2] or
+        None); a record's hull and approximation start at its point_offset."""
+        method = self.CHAIN[method] if isinstance(method, str) else int(method)
+        b, max_contours = table.shape[0], table.shape[1]
+        max_points = points.shape[1]
+        counts_per_frame = 1 if counts.dim() == 1 else 2
+        shapes = self.empty((b, max_contours, SHAPE_DTYPE.itemsize), torch.uint8)
+        hull_t = self.empty((b, max_points, 2), torch.int32) if hull else None
+        approx_t = self.empty((b, max_points, 2), torch.int32) if approx else None
+        check(lib.bv_contour_shapes(self.handle, ffi.cast("bv_contour *", table.data_ptr()),
+                                    ffi.cast("int32_t *", counts.data_ptr()), counts_per_frame,
+                                    ffi.cast("int32_t *", points.data_ptr()), b, max_contours, max_points, method,
+                                    float(approx_epsilon), float(approx_relative), ffi.cast("bv_shape *", shapes.data_ptr()),
+                                    ffi.cast("int32_t *", hull_t.data_ptr()) if hull else ffi.NULL,
+                                    ffi.cast("int32_t *", approx_t.data_ptr()) if approx else ffi.NULL))
+        return shapes, hull_t, approx_t
 
     def blobs_to_numpy(self, blobs, nb):
         """Device blob table -> list (per frame) of structured numpy arrays."""

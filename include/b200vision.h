@@ -301,6 +301,43 @@ typedef struct bv_rrect {
 int bv_min_area_rects(bv_ctx *ctx, const bv_contour *contours_dev, const int32_t *n_contours_dev,
                       const int32_t *points_dev, int batch, int max_contours, int max_points, bv_rrect *rects_dev);
 
+/* Shape descriptors of every record of a contour table, from bv_find_contours (any mode, NONE or SIMPLE:
+ * counts_per_frame = 2, n_contours_dev = its (n_outer, n_holes) pairs) or bv_outer_contours (SIMPLE,
+ * counts_per_frame = 1), with the same contours_dev / points_dev / max_contours / max_points.  method (bv_chain_approx)
+ * selects each record's vertex count: n_points (NONE) or n_simple (SIMPLE); counts_per_frame = 1 takes SIMPLE only
+ * (BV_ERR_INVALID otherwise).  shapes_dev: bv_shape[batch *
+ * max_contours], entry i belongs to record i; valid = 0 for records past the count or max_contours and for records
+ * whose vertices did not fit (point_offset < 0), and nothing else is written for them.
+ * hull_dev / approx_dev (optional, NULL skips; a NULL approx_dev skips the Douglas-Peucker work): int32[batch]
+ * [max_points][2], shaped as points_dev; a record's hull and approximation start at its own point_offset (both have at
+ * most as many vertices as the record; the rest of the record's slots in approx_dev are overwritten as scratch).
+ * Each record's approximation accuracy is eps = approx_epsilon + approx_relative * arc_length (double, no fused
+ * multiply-add), the value `k * cv2.arcLength(c, True)` gives a caller.  Exactness against cv2 4.13.0:
+ *   arc_length      cv2.arcLength(c, True): bit-exact (float32 steps, summed exactly in double)
+ *   hull, n_hull    cv2.convexHull(c) (clockwise=False): the same vertices in the same order; the same first vertex
+ *                   for every contour that visits no pixel twice (cv2's first vertex depends on the order its
+ *                   unstable sort leaves repeated pixels in; the library takes the first visit of each pixel)
+ *   rect            cv2.minAreaRect(c), hole borders included; outer records bit-equal to bv_min_area_rects
+ *   approx          cv2.approxPolyDP(c, eps, True): bit-exact (OpenCV 4.13's algorithm, which splits a slice at the
+ *                   point farthest from its chord segment, in the same double operations)
+ *   approx_convex   cv2.isContourConvex(approx): exact
+ *   circle          cv2.minEnclosingCircle(c): the exact circle of the hull in double, radius + 1e-4, rounded to
+ *                   float32; cv2 itself is within ~1.3e-4 px of it (stated tolerance 2e-3 px) */
+typedef struct bv_shape {
+    double arc_length;
+    float circle_cx, circle_cy, circle_r;
+    bv_rrect rect;
+    int32_t n_hull;
+    int32_t n_approx;
+    int32_t approx_convex;
+    int32_t valid;
+    int32_t reserved;
+} bv_shape;
+int bv_contour_shapes(bv_ctx *ctx, const bv_contour *contours_dev, const int32_t *n_contours_dev, int counts_per_frame,
+                      const int32_t *points_dev, int batch, int max_contours, int max_points, int method,
+                      double approx_epsilon, double approx_relative, bv_shape *shapes_dev, int32_t *hull_dev,
+                      int32_t *approx_dev);
+
 /* ---- resize / YOLO input ------------------------------------------------------------------ */
 /* cv2.resize(..., INTER_LINEAR) on uint8 (utils/transform.py:179, modules/preprocessor.py:136-143). */
 int bv_resize_linear(bv_ctx *ctx, const uint8_t *src_dev, int src_h, int src_w, uint8_t *dst_dev, int dst_h,
