@@ -162,7 +162,6 @@ struct bv_ctx {
     int lb_smem_set;     // same for letterbox_tma_kernel
     void *lb_cache;      // host copy of the letterbox descriptors whose tap table is on the device
     int lb_cache_n, lb_cache_ow, lb_cache_oh;
-    int chain_smem_set;  // largest dynamic shared-memory size already enabled for morph_chain_kernel
     int opt[BV_OPT_COUNT];  // tuning knobs, 0 = built-in default (bv_set_option)
     int *d_ivl_flag;
 };

@@ -13,6 +13,9 @@
 //     and an AND across 5 rows per 32 pixels; the whole mask of a 2208x1242 frame is 343 KB and
 //     lives in L2.  Used by the fused stage (stage.cu).
 //   * grey / multi-channel uint8 with an arbitrary SE given as horizontal runs (bv_morph).
+#include <mutex>
+#include <unordered_map>
+
 #include "morph.cuh"
 
 namespace bv {
@@ -169,45 +172,48 @@ static int morph_bits_basic(bv_ctx *ctx, const uint32_t *src, uint32_t *dst, uin
     return BV_OK;
 }
 
-int morph_bits_rect(bv_ctx *ctx, uint32_t *bits, uint32_t *tmp, uint32_t *tmp2, int batch, int height, int width, int op,
-                    int kw, int kh, int iterations) {
-    if (iterations < 1) return BV_OK;
-    if (kw == 1 && kh == 1) {  // identity element: dilate == erode == input, so the gradient is empty
-        if (op == BV_MORPH_GRADIENT)
-            BV_CUDA(cudaMemsetAsync(bits, 0, (size_t)batch * height * words_per_row(width) * 4, ctx->stream));
+// taps of a kw x kh rectangle applied `iterations` times, x-L .. x+R and y-U .. y+D, computed in 64 bits and clipped to the
+// frame: a tap that lies a whole width or height away from every pixel never reads the image, so the clip changes nothing
+static void rect_extents(int kw, int kh, int iterations, int height, int width, int &L, int &R, int &U, int &D) {
+    const long long ax = kw / 2, ay = kh / 2, n = iterations;
+    L = (int)min(ax * n, (long long)width - 1);
+    R = (int)min((kw - 1 - ax) * n, (long long)width - 1);
+    U = (int)min(ay * n, (long long)height - 1);
+    D = (int)min((kh - 1 - ay) * n, (long long)height - 1);
+}
+
+int morph_bits_rect(bv_ctx *ctx, uint32_t *bits, uint32_t *tmp, uint32_t *tmp2, uint32_t *tmp3, int batch, int height,
+                    int width, int op, int kw, int kh, int iterations) {
+    const size_t total = (size_t)batch * height * words_per_row(width);
+    // zero iterations or the identity element: dilate == erode == input, so the gradient is empty (cv2 4.13.0)
+    if (iterations < 1 || (kw == 1 && kh == 1)) {
+        if (op == BV_MORPH_GRADIENT) BV_CUDA(cudaMemsetAsync(bits, 0, total * 4, ctx->stream));
         return BV_OK;
     }
-    const int ax = kw / 2, ay = kh / 2;
-    // taps: x-ax .. x+(kw-1-ax) for erosion and dilation alike
-    const int eL = ax * iterations, eR = (kw - 1 - ax) * iterations, eU = ay * iterations, eD = (kh - 1 - ay) * iterations;
-    const int dL = eL, dR = eR, dU = eU, dD = eD;  // cv2 applies the same taps for dilation (probed, 4.13.0)
-    const size_t total = (size_t)batch * height * words_per_row(width);
+    // taps: x-L .. x+R, y-U .. y+D for erosion and dilation alike (cv2 does not mirror the element: probed, 4.13.0)
+    int L, R, U, D;
+    rect_extents(kw, kh, iterations, height, width, L, R, U, D);
     switch (op) {
         case BV_MORPH_ERODE:
-            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, true, eL, eR, eU, eD));
+            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, true, L, R, U, D));
             BV_CUDA(cudaMemcpyAsync(bits, tmp, total * 4, cudaMemcpyDeviceToDevice, ctx->stream));
             return BV_OK;
         case BV_MORPH_DILATE:
-            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, false, dL, dR, dU, dD));
+            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, false, L, R, U, D));
             BV_CUDA(cudaMemcpyAsync(bits, tmp, total * 4, cudaMemcpyDeviceToDevice, ctx->stream));
             return BV_OK;
         case BV_MORPH_OPEN:
-            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, true, eL, eR, eU, eD));
-            return morph_bits_basic(ctx, tmp, bits, tmp2, batch, height, width, false, dL, dR, dU, dD);
+            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, true, L, R, U, D));
+            return morph_bits_basic(ctx, tmp, bits, tmp2, batch, height, width, false, L, R, U, D);
         case BV_MORPH_CLOSE:
-            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, false, dL, dR, dU, dD));
-            return morph_bits_basic(ctx, tmp, bits, tmp2, batch, height, width, true, eL, eR, eU, eD);
-        case BV_MORPH_GRADIENT: {
-            // needs three images: bits (input), tmp (dilated), tmp2 (eroded); both basics must be single-pass
-            if (eL > 31 || eR > 31 || eU > 31 || eD > 31) {
-                set_error("binary gradient: structuring element too large");
-                return BV_ERR_UNSUPPORTED;
-            }
-            BV_TRY(morph_bits_basic(ctx, bits, tmp, nullptr, batch, height, width, false, dL, dR, dU, dD));
-            BV_TRY(morph_bits_basic(ctx, bits, tmp2, nullptr, batch, height, width, true, eL, eR, eU, eD));
+            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp2, batch, height, width, false, L, R, U, D));
+            return morph_bits_basic(ctx, tmp, bits, tmp2, batch, height, width, true, L, R, U, D);
+        case BV_MORPH_GRADIENT:
+            // bits (input), tmp (dilated), tmp2 (eroded); tmp3 is the ping-pong image of either basic's passes
+            BV_TRY(morph_bits_basic(ctx, bits, tmp, tmp3, batch, height, width, false, L, R, U, D));
+            BV_TRY(morph_bits_basic(ctx, bits, tmp2, tmp3, batch, height, width, true, L, R, U, D));
             BV_LAUNCH(ctx, bits_andnot_kernel, grid_for(ctx, total, 256, 8), 256, 0, tmp, tmp2, bits, total);
             return BV_OK;
-        }
         default: set_error("unknown morphology op %d", op); return BV_ERR_INVALID;
     }
 }
@@ -524,11 +530,13 @@ int morph_bits_chain(bv_ctx *ctx, const uint32_t *bits, uint32_t *dst_bits, uint
     MorphChain ch;
     memset(&ch, 0, sizeof(ch));
     for (int s = 0; s < n_steps; ++s) {
-        if (iters[s] < 1 || (kws[s] == 1 && khs[s] == 1 && ops[s] != BV_MORPH_GRADIENT)) continue;  // identity
-        if (ops[s] == BV_MORPH_GRADIENT) return BV_OK;
-        const int ax = kws[s] / 2, ay = khs[s] / 2;
-        const int L = ax * iters[s], R = (kws[s] - 1 - ax) * iters[s], U = ay * iters[s], D = (khs[s] - 1 - ay) * iters[s];
-        if (L > 31 || R > 31) return BV_OK;
+        if (ops[s] == BV_MORPH_GRADIENT) return BV_OK;   // three images: the step-by-step path (also at 0 iterations)
+        if (iters[s] < 1 || (kws[s] == 1 && khs[s] == 1)) continue;  // identity
+        const long long ax = kws[s] / 2, ay = khs[s] / 2, it = iters[s];
+        if (ax * it > 31 || (kws[s] - 1 - ax) * it > 31) return BV_OK;
+        const int L = (int)(ax * it), R = (int)((kws[s] - 1 - ax) * it);
+        if (ay * it > 256 || (khs[s] - 1 - ay) * it > 256) return BV_OK;   // more than the 256 rows a tile may have
+        const int U = (int)(ay * it), D = (int)((khs[s] - 1 - ay) * it);
         const int first_erode = (ops[s] == BV_MORPH_ERODE || ops[s] == BV_MORPH_OPEN) ? 1 : 0;
         const int n_el = (ops[s] == BV_MORPH_OPEN || ops[s] == BV_MORPH_CLOSE) ? 2 : 1;
         for (int e = 0; e < n_el; ++e) {
@@ -574,10 +582,18 @@ int morph_bits_chain(bv_ctx *ctx, const uint32_t *bits, uint32_t *dst_bits, uint
     const int tile_rows = rows - halo;
     const size_t smem = (size_t)2 * rows * wpr * sizeof(uint32_t);
     if (rows > 256 || smem > 200 * 1024) return BV_OK;
-    if (smem > 48 * 1024 && smem > (size_t)ctx->chain_smem_set) {
-        BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ctx->chain_smem_set = (int)smem;
+    if (smem > 48 * 1024) {
+        // the opt-in is an attribute of the kernel on the device, shared by every context of the process: it is only ever
+        // raised, so that a context's smaller launch cannot take away what another context's larger one relies on
+        static std::mutex mu;
+        static std::unordered_map<int, int> enabled;   // device -> bytes
+        std::lock_guard<std::mutex> lock(mu);
+        int &cur = enabled[ctx->device];
+        if ((int)smem > cur) {
+            BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            cur = (int)smem;
+        }
     }
     const int tiles = (height + tile_rows - 1) / tile_rows;
     if (ctx->opt[BV_OPT_MORPH_VARIANT] == 2)
@@ -596,7 +612,8 @@ int morph_bits_chain(bv_ctx *ctx, const uint32_t *bits, uint32_t *dst_bits, uint
 constexpr int kMaxRuns = 256;
 struct RunList {
     int n;
-    short dy[kMaxRuns], x0[kMaxRuns], x1[kMaxRuns];  // taps (x + x0 .. x + x1, y + dy)
+    short dy[kMaxRuns];
+    int x0[kMaxRuns], x1[kMaxRuns];  // taps (x + x0 .. x + x1, y + dy); a rectangle's row run spans up to the frame width
 };
 
 template <bool ERODE>
@@ -697,25 +714,34 @@ static int grey_basic(bv_ctx *ctx, const uint8_t *src, uint8_t *dst, uint8_t *t1
         return BV_OK;
     }
     if (se.rect) {
-        // separable, and n iterations of a rectangle == one rectangle with n-fold extents
-        const int ax = se.kw / 2, ay = se.kh / 2;
-        int L = ax * iterations, R = (se.kw - 1 - ax) * iterations, U = ay * iterations, D = (se.kh - 1 - ay) * iterations;
+        // separable, and n iterations of a rectangle == one rectangle with n-fold extents, clipped to the frame
+        int L, R, U, D;
+        rect_extents(se.kw, se.kh, iterations, height, width, L, R, U, D);
         RunList h, v;
         h.n = 1;
         h.dy[0] = 0;
-        h.x0[0] = (short)-L;
-        h.x1[0] = (short)R;
-        if (U + D + 1 > kMaxRuns) {
-            set_error("bv_morph: rectangle too tall after iterations");
-            return BV_ERR_UNSUPPORTED;
-        }
-        v.n = U + D + 1;
-        for (int k = 0; k < v.n; ++k) {
-            v.dy[k] = (short)(k - U);
-            v.x0[k] = v.x1[k] = 0;
-        }
+        h.x0[0] = -L;
+        h.x1[0] = R;
         BV_TRY(launch_grey(ctx, src, t1, height, width, cn, total, erode, h));
-        return launch_grey(ctx, t1, dst, height, width, cn, total, erode, v);
+        // the column taps y-U .. y+D in passes of at most kMaxRuns rows (U + D = sum of the passes' u + d): with out-of-image
+        // taps ignored, erosions (dilations) by segments that contain their anchor compose into one by the summed segment.
+        // Pass k of P writes dst when (P - k) is even, t2 otherwise, so the last pass lands in dst.
+        const int passes = U + D == 0 ? 1 : (U + D + kMaxRuns - 2) / (kMaxRuns - 1);
+        const uint8_t *cur = t1;
+        for (int k = 1; k <= passes; ++k) {
+            const int u = min(U, kMaxRuns - 1), d = min(D, kMaxRuns - 1 - u);
+            U -= u;
+            D -= d;
+            v.n = u + d + 1;
+            for (int j = 0; j < v.n; ++j) {
+                v.dy[j] = (short)(j - u);
+                v.x0[j] = v.x1[j] = 0;
+            }
+            uint8_t *out = ((passes - k) % 2 == 0) ? dst : t2;
+            BV_TRY(launch_grey(ctx, cur, out, height, width, cn, total, erode, v));
+            cur = out;
+        }
+        return BV_OK;
     }
     const RunList &runs = erode ? se.erode_runs : se.dilate_runs;
     const uint8_t *cur = src;
@@ -740,8 +766,12 @@ extern "C" int bv_morph(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, i
     BV_REQUIRE(op >= BV_MORPH_ERODE && op <= BV_MORPH_GRADIENT, "unknown morphology op");
     BV_CUDA(cudaSetDevice(ctx->device));
     const size_t total = (size_t)batch * height * width * channels;
-    if (iterations < 1) {  // cv2 treats iterations == 0 as "no-op copy"
-        if (src_dev != dst_dev) BV_CUDA(cudaMemcpyAsync(dst_dev, src_dev, total, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (iterations < 0) iterations = 1;   // cv2 reads a negative count as 1 (probed, 4.13.0)
+    if (iterations == 0) {                 // cv2: the source unchanged, and for GRADIENT (dilate - erode of nothing) zeros
+        if (op == BV_MORPH_GRADIENT)
+            BV_CUDA(cudaMemsetAsync(dst_dev, 0, total, ctx->stream));
+        else if (src_dev != dst_dev)
+            BV_CUDA(cudaMemcpyAsync(dst_dev, src_dev, total, cudaMemcpyDeviceToDevice, ctx->stream));
         return BV_OK;
     }
     static thread_local SeInfo se;

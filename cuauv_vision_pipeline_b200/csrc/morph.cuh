@@ -14,9 +14,10 @@ int mask_to_bits(bv_ctx *ctx, const uint8_t *mask, uint32_t *bits, int batch, in
 int bits_to_mask(bv_ctx *ctx, const uint32_t *bits, uint8_t *mask, int batch, int height, int width);
 
 // One bv_morph_op with a kw x kh rectangle (anchor = centre) on bit-packed images.  `bits` holds
-// the input and receives the result; `tmp` is a same-sized scratch image.
-int morph_bits_rect(bv_ctx *ctx, uint32_t *bits, uint32_t *tmp, uint32_t *tmp2, int batch, int height, int width, int op,
-                    int kw, int kh, int iterations);
+// the input and receives the result; `tmp`, `tmp2` and `tmp3` are same-sized scratch images.  Extents
+// over 31 px take several passes; iterations < 1 is the identity, except for GRADIENT (all zero, as cv2).
+int morph_bits_rect(bv_ctx *ctx, uint32_t *bits, uint32_t *tmp, uint32_t *tmp2, uint32_t *tmp3, int batch, int height,
+                    int width, int op, int kw, int kh, int iterations);
 
 // The whole list of steps in one launch (tile + halo in shared memory), writing the final bits
 // (dst_bits, may be null, must differ from bits) and/or the uint8 mask (may be null).  *done = false

@@ -43,7 +43,7 @@ struct StageTail {
     const bv_stage_desc *desc;
     int height, width;
     bool bits_direct, want_label;
-    uint32_t *bits, *tmp, *tmp2;   // whole batch
+    uint32_t *bits, *tmp, *tmp2, *tmp3;   // whole batch
     const uint8_t *thr_mask;       // thresholded uint8 mask when the bits do not come straight from the pixel pass
     uint8_t *mask;                 // caller's mask (may be null)
     int32_t *labels;
@@ -56,7 +56,7 @@ struct StageTail {
     int run(bv_ctx *c, int f0, int nf) {
         ++calls;
         const size_t fw = bits_frame_words(height, width), fpx = (size_t)height * width;
-        uint32_t *b = bits + f0 * fw, *t = tmp + f0 * fw, *t2 = tmp2 + f0 * fw;
+        uint32_t *b = bits + f0 * fw, *t = tmp + f0 * fw, *t2 = tmp2 + f0 * fw, *t3 = tmp3 + f0 * fw;
         uint8_t *m = mask ? mask + f0 * fpx : nullptr;
         if (!bits_direct) BV_TRY(mask_to_bits(c, thr_mask + f0 * fpx, b, nf, height, width));
         const uint32_t *res = b;
@@ -68,7 +68,7 @@ struct StageTail {
                 if (want_label) res = t;
             } else {
                 for (int i = 0; i < desc->n_morph; ++i)
-                    BV_TRY(morph_bits_rect(c, b, t, t2, nf, height, width, desc->morph_op[i], desc->morph_kw[i], desc->morph_kh[i],
+                    BV_TRY(morph_bits_rect(c, b, t, t2, t3, nf, height, width, desc->morph_op[i], desc->morph_kw[i], desc->morph_kh[i],
                                            desc->morph_iters[i]));
                 if (m) BV_TRY(bits_to_mask(c, b, m, nf, height, width));
             }
@@ -144,10 +144,11 @@ int stage_run(bv_ctx *ctx, const bv_stage_desc *desc, const uint8_t *src, int ba
     if (need_bits) {
         const size_t words = (size_t)batch * bits_frame_words(height, width);
         BV_TRY(ensure_scratch(ctx, SCR_BITS_A, words * 4));
-        BV_TRY(ensure_scratch(ctx, SCR_BITS_B, words * 8));
+        BV_TRY(ensure_scratch(ctx, SCR_BITS_B, words * 12));   // tmp, tmp2, tmp3
         tail.bits = (uint32_t *)ctx->scratch[SCR_BITS_A];
         tail.tmp = (uint32_t *)ctx->scratch[SCR_BITS_B];
         tail.tmp2 = tail.tmp + words;
+        tail.tmp3 = tail.tmp2 + words;
         const bool aligned = host_aligned16(src) && (!balanced || host_aligned16(balanced)) &&
                              (!converted || host_aligned16(converted)) && (!mask || host_aligned16(mask));
         tail.bits_direct = aligned && (width % 16 == 0) && !tiled;

@@ -105,7 +105,8 @@ typedef struct bv_balance_stats {
 } bv_balance_stats;
 
 /* One labelled blob: exact integer raster moments up to third order and the bounding box
- * (inclusive).  Labels are 1..n in raster order of each blob's first pixel.  Plays the role of
+ * (inclusive), exact while every sum fits int64 (the widest fully set row whose m30 fits has 77 936 px, and so has the
+ * tallest column for m03).  Labels are 1..n in raster order of each blob's first pixel.  Plays the role of
  * outer_contours + contour_centroid + contour_area (utils/feature.py:5-21,240-265). */
 typedef struct bv_blob {
     int64_t m00, m10, m01, m20, m11, m02, m30, m21, m12, m03;
@@ -212,8 +213,12 @@ int bv_color_distance_f32(bv_ctx *ctx, const uint8_t *const *planes_dev, size_t 
 int bv_select_kth_f32(bv_ctx *ctx, const float *values_dev, size_t n, size_t k, float *value_host);
 
 /* ---- morphology ------------------------------------------------------------------------------ */
-/* se_host: kh*kw bytes (non-zero = member), anchor = centre; channels 1 or 3 (per channel).
- * Border handling is cv2's default (BORDER_CONSTANT with morphologyDefaultBorderValue). */
+/* se_host: kh*kw bytes (non-zero = member), anchor = centre; channels 1..4 (per channel); src_dev == dst_dev is allowed.
+ * Border handling is cv2's default (BORDER_CONSTANT with morphologyDefaultBorderValue).  Iterations as cv2 counts them:
+ * a negative count is read as 1; 0 returns the source, and for GRADIENT all zeros.  A rectangle of any size and count is
+ * computed (its n iterations are one rectangle with n-fold extents); any other element may have at most 256 horizontal
+ * runs (BV_ERR_UNSUPPORTED beyond).  In bv_stage_desc a negative count is rejected (BV_ERR_INVALID) and 0 follows the
+ * same rule. */
 int bv_morph(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width,
              int channels, int op, const uint8_t *se_host, int kw, int kh, int iterations);
 
