@@ -27,15 +27,6 @@
 
 namespace bv {
 
-__device__ __forceinline__ int find_root(int *parent, int a) {
-    int p = parent[a];
-    while (p != a) {
-        a = p;
-        p = parent[a];
-    }
-    return a;
-}
-
 __device__ __forceinline__ int find_compress(int *parent, int a) {
     const int a0 = a;
     int p = parent[a];
@@ -64,27 +55,6 @@ __device__ void union_nodes(int *parent, int a, int b) {
             done = true;
         }
     } while (!done);
-}
-
-// first bit of the run of ones containing bit `pos` of w (w has bit pos set)
-__device__ __forceinline__ int run_start(uint32_t w, int pos) {
-    const uint32_t zeros_below = ~w & ((pos == 0) ? 0u : (0xFFFFFFFFu >> (32 - pos)));
-    return zeros_below ? 32 - __clz(zeros_below) : 0;
-}
-
-struct WordPos {
-    int wx, y;
-    uint32_t row;  // frame * height + y
-};
-
-// 32-bit index math throughout the word-indexed kernels (64-bit div/mod costs ~10x; the host
-// refuses batches of 2^31 words or more)
-__device__ __forceinline__ WordPos word_pos(uint32_t i, int wpr, int height) {
-    WordPos p;
-    p.wx = (int)(i % (uint32_t)wpr);
-    p.row = i / (uint32_t)wpr;
-    p.y = (int)(p.row % (uint32_t)height);
-    return p;
 }
 
 __global__ void __launch_bounds__(256) ccl_init_kernel(const uint32_t *__restrict__ bits, int *__restrict__ parent,
@@ -569,6 +539,15 @@ static LabelScratch label_scratch_slice(const LabelScratch &ls, int f0, int heig
 static int label_bits_ex(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int batch, int height, int width,
                          bv_blob *blobs, int max_blobs, int32_t *n_blobs, int *root_px, int max_roots, const LabelScratch &sc,
                          uint32_t *outer = nullptr);
+
+int union_bits(bv_ctx *ctx, const uint32_t *bits, int batch, int height, int width, const LabelScratch &ls) {
+    const int wpr = words_per_row(width);
+    const size_t total_words = (size_t)batch * height * wpr;
+    const int gw = grid_for(ctx, total_words, 256, 8);
+    BV_LAUNCH(ctx, ccl_init_kernel, gw, 256, 0, bits, ls.parent, height, width, wpr, (uint32_t)total_words);
+    BV_LAUNCH(ctx, ccl_merge_kernel<true>, gw, 256, 0, bits, ls.parent, height, width, wpr, (uint32_t)total_words);
+    return BV_OK;
+}
 
 int label_bits(bv_ctx *ctx, const uint32_t *bits, int32_t *labels, int batch, int height, int width, bv_blob *blobs,
                int max_blobs, int32_t *n_blobs) {

@@ -53,22 +53,7 @@ __global__ void __launch_bounds__(256) bits_to_mask_kernel(const uint32_t *__res
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total_words; i += stride) {
         const int wx = (int)(i % (uint32_t)wpr);
         const uint32_t row = i / (uint32_t)wpr;
-        uint8_t *p = mask + (size_t)row * width + (size_t)wx * 32;
-        const int n = min(32, width - wx * 32);
-        const uint32_t w = bits[i];
-        if (n == 32 && ((reinterpret_cast<uintptr_t>(p) & 15) == 0)) {
-            uint32_t v[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-                const uint32_t nib = (w >> (4 * k)) & 0xF;
-                v[k] = ((nib & 1) * 0xFFu) | (((nib >> 1) & 1) * 0xFF00u) | (((nib >> 2) & 1) * 0xFF0000u) |
-                       (((nib >> 3) & 1) * 0xFF000000u);
-            }
-            st_stream(reinterpret_cast<uint4 *>(p), make_uint4(v[0], v[1], v[2], v[3]));
-            st_stream(reinterpret_cast<uint4 *>(p) + 1, make_uint4(v[4], v[5], v[6], v[7]));
-        } else {
-            for (int k = 0; k < n; ++k) p[k] = ((w >> k) & 1) ? 255 : 0;
-        }
+        store_mask_word(mask + (size_t)row * width + (size_t)wx * 32, min(32, width - wx * 32), bits[i]);
     }
 }
 

@@ -1,8 +1,9 @@
 """Blob extraction: the role of the reference's outer_contours / contour_centroid / contour_area
-(utils/feature.py:5-21,240-265) as connected-component labelling with exact raster moments."""
+(utils/feature.py:5-21,240-265) as connected-component labelling with exact raster moments; every border with its
+hierarchy and shape descriptors; and cv2.Canny edges that feed them without leaving the device."""
 import numpy as np
 
-from ._host import ctx_for, to_device, is_device, release_to_caller
+from ._host import ctx_for, to_device, is_device, release_to_caller, like_input
 
 
 class Blob(dict):
@@ -172,6 +173,15 @@ def _attach_shapes(ctx, out, records, table, counts, pts, method, approx_epsilon
         c["approx_convex"] = bool(s["approx_convex"])
         c["min_enclosing_circle"] = ((float(s["circle_cx"]), float(s["circle_cy"])), float(s["circle_r"]))
         c["min_area_rect"] = ((float(r["cx"]), float(r["cy"])), (float(r["width"]), float(r["height"])), float(r["angle"]))
+
+
+def canny(image, threshold1, threshold2, apertureSize=3, L2gradient=False):
+    """cv2.Canny(image, threshold1, threshold2, apertureSize=apertureSize, L2gradient=L2gradient) on the GPU, bit-exact:
+    uint8 0/255 edges of a grey [H,W] or BGR [H,W,3] image (or a batch [B,H,W] / [B,H,W,3] of them).  Numpy in gives
+    numpy out; a CUDA tensor in gives a CUDA tensor out without leaving the device, so
+    `find_contours(canny(frame, ...))` runs on the device throughout."""
+    ctx = ctx_for(image)
+    return like_input(ctx, image, ctx.canny(to_device(ctx, image), threshold1, threshold2, apertureSize, L2gradient))
 
 
 def _contour_moments(c):

@@ -284,6 +284,25 @@ class Context:
                            ffi.from_buffer("uint8_t[]", kernel), kw, kh, int(iterations)))
         return dst
 
+    def canny(self, src, threshold1, threshold2, aperture_size=3, l2_gradient=False):
+        """cv2.Canny(src, threshold1, threshold2, apertureSize=aperture_size, L2gradient=l2_gradient) of a device image
+        [H,W], [H,W,3], [B,H,W] or [B,H,W,3] (a rank-3 tensor whose last dimension is 3 is one BGR frame) -> uint8 0/255
+        [.., H, W], bit-exact (bv_canny).  BVError for an aperture other than 3, 5 or 7, as cv2 raises."""
+        self._src(src)
+        if src.dim() == 2:
+            b, h, w, c = 1, src.shape[0], src.shape[1], 1
+        elif src.dim() == 3:
+            b, h, w, c = (1, src.shape[0], src.shape[1], 3) if src.shape[2] == 3 else (src.shape[0], src.shape[1],
+                                                                                        src.shape[2], 1)
+        elif src.dim() == 4 and src.shape[3] in (1, 3):
+            b, h, w, c = src.shape
+        else:
+            raise BVError(-1, "canny takes [H,W], [H,W,3], [B,H,W] or [B,H,W,3]")
+        dst = self.empty((b, h, w) if src.dim() == 4 or (src.dim() == 3 and c == 1) else (h, w))
+        check(lib.bv_canny(self.handle, _u8ptr(src), _u8ptr(dst), b, h, w, c, float(threshold1), float(threshold2),
+                           int(aperture_size), 1 if l2_gradient else 0))
+        return dst
+
     def color_balance(self, src, want_stats=False, **flags):
         b, h, w, c = self._bhw(src)
         if c != 3:

@@ -222,6 +222,24 @@ int bv_select_kth_f32(bv_ctx *ctx, const float *values_dev, size_t n, size_t k, 
 int bv_morph(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width,
              int channels, int op, const uint8_t *se_host, int kw, int kh, int iterations);
 
+/* ---- edges ------------------------------------------------------------------------------------ */
+/* cv2.Canny(src, threshold1, threshold2, apertureSize=aperture_size, L2gradient=l2_gradient) of every frame, bit-exact
+ * against OpenCV 4.13.0 (a module's edge detection, cv2.Canny on the host, moved to the device).  src_dev: uint8
+ * [batch,H,W,channels], channels 1 or 3; dst_dev: uint8 [batch,H,W] of 0/255.  The rules:
+ *   1. dx, dy = Sobel(src, CV_16S, ksize = aperture_size, BORDER_REPLICATE) of each channel; aperture 7 scales them by
+ *      1/16 (rounded half to even) and divides both thresholds by 16 first.
+ *   2. magnitude |dx| + |dy| (L1) or dx^2 + dy^2 (L2); on 3 channels the channel with the largest magnitude (the first
+ *      on a tie) gives the pixel's magnitude, dx and dy.
+ *   3. L2: each threshold becomes min(t, 32767), squared when positive; low > high swaps them; both are floored
+ *      (INT_MIN for NaN or beyond int32, as cvFloor on x86-64).
+ *   4. non-maximum suppression across the gradient direction (tan 22.5 deg in 15-bit fixed point; magnitude 0 outside
+ *      the frame): a kept pixel with magnitude > low is a candidate, a candidate with magnitude > high is strong.
+ *   5. 255 on every candidate whose 8-connected component of candidates holds a strong pixel (union-find, not a stack).
+ * Frames are independent.  BV_ERR_INVALID (as cv2 raises) for an aperture other than 3, 5 or 7; also for overlapping
+ * src / dst ranges and for frames or batches past bv_label's 32-bit index limits. */
+int bv_canny(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width, int channels,
+             double threshold1, double threshold2, int aperture_size, int l2_gradient);
+
 /* ---- connected components + moments ------------------------------------------------------- */
 /* 8-connected labelling of mask != 0.  labels_dev: int32[batch,H,W] (0 = background).
  * blobs_dev: bv_blob[batch * max_blobs] (may be NULL), n_blobs_dev: int32[batch] total blob
