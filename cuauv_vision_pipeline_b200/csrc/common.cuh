@@ -115,6 +115,10 @@ enum ScratchSlot {
     SCR_HOST1_NBLOBS,
     SCR_IVL_FRAMES,     // hue-interval table composed with every frame's S / V stretch tables (balance.cu)
     SCR_INGEST,         // landing buffer of 4-channel frames ingested from a shared-memory ring (ingest.cu)
+    SCR_HOUGH_TAB,      // trig table of the Hough transform, then per-frame edge and peak counts (hough.cu)
+    SCR_HOUGH_ACC,      // int32 Hough accumulators of one group of frames
+    SCR_HOUGH_KEYS,     // peak keys of one group of frames, two buffers for the radix sort
+    SCR_HOUGH_EDGES,    // edge-pixel lists of one group of frames (+ their values with use_edgeval)
     SCR_COUNT
 };
 

@@ -1,9 +1,9 @@
 """Blob extraction: the role of the reference's outer_contours / contour_centroid / contour_area
 (utils/feature.py:5-21,240-265) as connected-component labelling with exact raster moments; every border with its
-hierarchy and shape descriptors; and cv2.Canny edges that feed them without leaving the device."""
+hierarchy and shape descriptors; and cv2.Canny edges and cv2.HoughLines lines of them without leaving the device."""
 import numpy as np
 
-from ._host import ctx_for, to_device, is_device, release_to_caller, like_input
+from ._host import ctx_for, to_device, is_device, release_to_caller, like_input, on_ctx_stream
 
 
 class Blob(dict):
@@ -182,6 +182,38 @@ def canny(image, threshold1, threshold2, apertureSize=3, L2gradient=False):
     `find_contours(canny(frame, ...))` runs on the device throughout."""
     ctx = ctx_for(image)
     return like_input(ctx, image, ctx.canny(to_device(ctx, image), threshold1, threshold2, apertureSize, L2gradient))
+
+
+def hough_lines(image, rho, theta, threshold, srn=0, stn=0, min_theta=0, max_theta=np.pi, use_edgeval=False,
+                votes=False, max_lines=4096):
+    """cv2.HoughLines(image, rho, theta, threshold, srn=srn, stn=stn, min_theta=min_theta, max_theta=max_theta) on the
+    GPU, bit-exact: float32 [N,1,2] (rho, theta) in cv2's order, or None when there is no line.  With votes=True it is
+    cv2.HoughLinesWithAccumulator(..., use_edgeval=use_edgeval): [N,1,3] with the votes.  image: uint8 [H,W], or a
+    batch [B,H,W] for a list of one result per frame.  Numpy in gives numpy out; a CUDA tensor in gives CUDA tensors out,
+    so `hough_lines(canny(frame, ...), ...)` leaves the device only for the line counts.  max_lines is a first guess: when
+    a frame has more lines, the call is repeated once with room for all of them.  The multi-scale transform (srn or stn
+    other than 0) is not served: ValueError."""
+    if srn or stn:
+        raise ValueError("the multi-scale Hough transform (srn, stn != 0) is not served")
+    ctx = ctx_for(image)
+    dev = to_device(ctx, image)
+    args = (rho, theta, threshold, min_theta, max_theta, use_edgeval)
+    lines, n_lines = ctx.hough_lines(dev, *args, max_lines=max_lines)
+    counts = np.atleast_1d(ctx.download(n_lines))
+    if counts.max() > max_lines:
+        max_lines = int(counts.max())
+        lines, n_lines = ctx.hough_lines(dev, *args, max_lines=max_lines)
+    cols = 3 if votes else 2
+    counts = [int(n) for n in counts]
+    frames = lines.reshape(len(counts), max_lines, 3)
+    if is_device(image):
+        with on_ctx_stream(ctx):
+            out = [frames[k, :n, :cols].reshape(n, 1, cols).contiguous() if n else None for k, n in enumerate(counts)]
+        out = [release_to_caller(ctx, t) for t in out]
+    else:
+        host = ctx.download(frames[:, :max(counts), :cols])
+        out = [host[k, :n].reshape(n, 1, cols).copy() if n else None for k, n in enumerate(counts)]
+    return out if len(image.shape) == 3 else out[0]
 
 
 def _contour_moments(c):

@@ -5,6 +5,7 @@ PyTorch is used only to own device memory and to copy between host and device
 CUDA kernel inside libb200vision.so.  There is no CPU path: creating a Context without a usable
 CUDA device raises BVError.
 """
+import math
 import threading
 
 import numpy as np
@@ -302,6 +303,27 @@ class Context:
         check(lib.bv_canny(self.handle, _u8ptr(src), _u8ptr(dst), b, h, w, c, float(threshold1), float(threshold2),
                            int(aperture_size), 1 if l2_gradient else 0))
         return dst
+
+    def hough_lines(self, src, rho, theta, threshold, min_theta=0.0, max_theta=math.pi, use_edgeval=False,
+                    max_lines=4096):
+        """cv2.HoughLinesWithAccumulator(src, rho, theta, threshold, min_theta=, max_theta=, use_edgeval=) of a device
+        image [H,W] or batch [B,H,W] (bv_hough_lines) -> (lines float32 [.., max_lines, 3] = rho, theta, votes in cv2's
+        order, n_lines int32 [..]: the lines each frame has, which may exceed max_lines).  BVError where cv2 raises
+        (rho <= 0, theta <= 0, min_theta > max_theta)."""
+        self._src(src)
+        if src.dim() == 2:
+            b, (h, w) = 1, src.shape
+        elif src.dim() == 3:
+            b, h, w = src.shape
+        else:
+            raise BVError(-1, "hough_lines takes [H,W] or [B,H,W]")
+        lines = self.empty((b, int(max_lines), 3), torch.float32)
+        n_lines = self.empty((b,), torch.int32)
+        check(lib.bv_hough_lines(self.handle, _u8ptr(src), b, h, w, float(rho), float(theta), int(threshold),
+                                 float(min_theta), float(max_theta), 1 if use_edgeval else 0,
+                                 ffi.cast("float *", lines.data_ptr()), int(max_lines),
+                                 ffi.cast("int32_t *", n_lines.data_ptr())))
+        return (lines[0], n_lines[0]) if src.dim() == 2 else (lines, n_lines)
 
     def color_balance(self, src, want_stats=False, **flags):
         b, h, w, c = self._bhw(src)

@@ -240,6 +240,37 @@ int bv_morph(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, i
 int bv_canny(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width, int channels,
              double threshold1, double threshold2, int aperture_size, int l2_gradient);
 
+/* ---- straight lines --------------------------------------------------------------------------- */
+/* cv2.HoughLines(src, rho, theta, threshold, min_theta=, max_theta=) of every frame, and with the votes
+ * cv2.HoughLinesWithAccumulator(..., use_edgeval=), bit-exact against OpenCV 4.13.0 (the standard transform; srn = stn
+ * = 0).  src_dev: uint8 [batch,H,W], typically an edge map; lines_dev: float32 [batch][max_lines][3] = (rho, theta,
+ * votes) of each frame's first max_lines lines; n_lines_dev: int32 [batch], the lines each frame has (may exceed
+ * max_lines: call again with room for them).  The rules:
+ *   1. rho and theta are taken as float32; irho = 1.0f / rho.
+ *   2. numangle = floor((max_theta - min_theta) / theta) + 1 in double, less one when numangle > 1 and
+ *      |pi - (numangle - 1) * theta| < theta / 2.
+ *   3. numrho = cvRound((2 * (W + H) + 1) / rho), float32 division, half to even.
+ *   4. the trig table, built on the host: ang = float32(min_theta); tabSin[n] = float32(sin(double(ang)) * irho),
+ *      tabCos[n] likewise; then ang += theta in float32.
+ *   5. every non-zero pixel (x column, y row) adds 1 (its value with use_edgeval) to the int32 accumulator
+ *      [numangle + 2][numrho + 2] (zero border) at flat index (n + 1) * (numrho + 2) + r + 1,
+ *      r = cvRound(x * tabCos[n] + y * tabSin[n]) + (numrho - 1) / 2: two float32 products and a float32 sum, each
+ *      rounded (no FMA), rounded half to even, integer division.
+ *   6. a bin is a line when votes > threshold, > the bin before and >= the bin after along rho, > the bin before and
+ *      >= the bin after along theta (the border zeros take part).
+ *   7. lines are ordered by votes descending, then by flat index ascending (cv2 returns them all).
+ *   8. rho = float32(r - (numrho - 1) / 2) * rho (integer division); theta = float32(min_theta) + float32(n) * theta,
+ *      each operation rounded to float32; votes = float32(votes).
+ *   9. cv2 returns None when there is no line, else [N,1,2] ([N,1,3] with the votes): the Python wrapper does that.
+ *  10. BV_ERR_INVALID where cv2 raises: rho <= 0, theta <= 0 (as float32), min_theta > max_theta; also for non-finite
+ *      rho, theta, min_theta or max_theta, for overlapping src / lines / n_lines ranges, for H or W above 65535, for
+ *      accumulators of 2^31 bins or more, and with use_edgeval when 255 * H * W passes INT32_MAX.  The multi-scale
+ *      transform (srn, stn) is not served.
+ * Frames are independent; the result does not depend on the order of any atomic operation. */
+int bv_hough_lines(bv_ctx *ctx, const uint8_t *src_dev, int batch, int height, int width, double rho, double theta,
+                   int threshold, double min_theta, double max_theta, int use_edgeval, float *lines_dev, int max_lines,
+                   int32_t *n_lines_dev);
+
 /* ---- connected components + moments ------------------------------------------------------- */
 /* 8-connected labelling of mask != 0.  labels_dev: int32[batch,H,W] (0 = background).
  * blobs_dev: bv_blob[batch * max_blobs] (may be NULL), n_blobs_dev: int32[batch] total blob
