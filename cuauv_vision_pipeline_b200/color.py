@@ -1,5 +1,7 @@
 """GPU mirror of the reference's utils/color.py (same function names, arguments and return
 shapes).  Citations are to /root/reference/utils/color.py."""
+import math
+
 import numpy as np
 
 from ._host import ctx_for, to_device, like_input
@@ -91,6 +93,81 @@ def _thresh(kind, maxval=255):
         mv = maxval if maxval is not None else 0
         return like_input(ctx, mat, ctx.threshold(to_device(ctx, mat), threshold, mv, kind))
     return fn
+
+
+# cv2's constants, so that callers of threshold / adaptive_threshold do not need OpenCV
+THRESH_BINARY, THRESH_BINARY_INV, THRESH_TRUNC, THRESH_TOZERO, THRESH_TOZERO_INV = 0, 1, 2, 3, 4
+THRESH_OTSU, THRESH_TRIANGLE = 8, 16
+ADAPTIVE_THRESH_MEAN_C, ADAPTIVE_THRESH_GAUSSIAN_C = 0, 1
+_INT_MIN = -2 ** 31
+
+
+def _cvt_si32(v):
+    """x86-64's double -> int32 conversion under cvRound: half to even, INT_MIN where the value has no int32."""
+    if not math.isfinite(v):
+        return _INT_MIN
+    r = round(v)
+    return r if _INT_MIN <= r < 2 ** 31 else _INT_MIN
+
+
+def _cv_floor(v):
+    """cvFloor as cv2.threshold reads its threshold: INT_MIN where the floor has no int32."""
+    if not math.isfinite(v):
+        return _INT_MIN
+    f = math.floor(v)
+    return f if _INT_MIN <= f < 2 ** 31 else _INT_MIN
+
+
+def _is_batch(shape):
+    return len(shape) == 4 or (len(shape) == 3 and shape[-1] != 3)
+
+
+def _grey_only(mat, what):
+    shape = tuple(mat.shape)
+    if not (len(shape) == 2 or len(shape) == 3 and shape[-1] != 3 or len(shape) == 4 and shape[-1] == 1):
+        raise ValueError("%s takes a grey frame [H,W] or a batch [B,H,W] / [B,H,W,1], not %r" % (what, shape))
+
+
+def threshold(mat, thresh, maxval, type):  # noqa: A002 (cv2's argument names)
+    """cv2.threshold(mat, thresh, maxval, type) on the GPU -> (retval, dst).  type is a base type (THRESH_BINARY ..
+    THRESH_TOZERO_INV), optionally with THRESH_OTSU or THRESH_TRIANGLE, which compute each frame's threshold on the device
+    (bv_threshold_auto, bit-exact; where two Otsu thresholds score exactly the same, the one cv2's own loop picks, which
+    cv2's IPP path, taken with its default optimisations, may not) and ignore `thresh`.  mat: [H,W] or a BGR [H,W,3]
+    (base types only), or a batch [B,H,W] / [B,H,W,1]; retval is a float for one frame and a float64 array of one value per frame for a batch.  Base
+    types follow cv2's 8-bit rules: retval = cvFloor(thresh), maxval rounded half to even and saturated.  Numpy in gives
+    numpy out; a CUDA tensor in gives a CUDA tensor out (the thresholds come back in one small download)."""
+    base, auto = type & 7, type & (THRESH_OTSU | THRESH_TRIANGLE)
+    if base > THRESH_TOZERO_INV or type & ~(7 | THRESH_OTSU | THRESH_TRIANGLE):
+        raise ValueError("unknown threshold type %r" % type)
+    if auto == THRESH_OTSU | THRESH_TRIANGLE:
+        raise ValueError("THRESH_OTSU and THRESH_TRIANGLE cannot be combined")
+    shape = tuple(mat.shape)
+    ctx = ctx_for(mat)
+    if auto:
+        _grey_only(mat, "threshold with THRESH_OTSU / THRESH_TRIANGLE")
+        dst, th = ctx.threshold_auto(to_device(ctx, mat), maxval, base, "otsu" if auto == THRESH_OTSU else "triangle")
+        ret = ctx.download(th)
+        retval = ret if _is_batch(shape) else float(ret)
+    else:
+        ithresh = _cv_floor(float(thresh))
+        imax = _cvt_si32(float(maxval))
+        # every uint8 compares the same against any threshold below 0 or from 255 up
+        dst = ctx.threshold(to_device(ctx, mat), min(max(ithresh, -1), 255), min(max(imax, 0), 255),
+                            ("binary", "binary_inv", "trunc", "tozero", "tozero_inv")[base])
+        retval = np.full(shape[0], float(ithresh)) if _is_batch(shape) else float(ithresh)
+    return retval, like_input(ctx, mat, dst)
+
+
+def adaptive_threshold(mat, maxValue, adaptiveMethod, thresholdType, blockSize, C):  # noqa: N803 (cv2's names)
+    """cv2.adaptiveThreshold(mat, maxValue, adaptiveMethod, thresholdType, blockSize, C) on the GPU
+    (bv_adaptive_threshold): ADAPTIVE_THRESH_MEAN_C bit-exact, ADAPTIVE_THRESH_GAUSSIAN_C bit-exact for blockSize <= 9
+    and above it different only where the mean lies within 1e-3 of a half-integer (cv2's own summation order varies).  mat: a grey frame [H,W] or a batch [B,H,W] / [B,H,W,1]; a BGR
+    frame is refused as cv2 refuses it.  Numpy in gives numpy out; a CUDA tensor in gives a CUDA tensor out, so
+    `feature.find_contours(adaptive_threshold(frame, ...))` runs on the device throughout."""
+    _grey_only(mat, "adaptive_threshold")
+    ctx = ctx_for(mat)
+    return like_input(ctx, mat, ctx.adaptive_threshold(to_device(ctx, mat), maxValue, int(adaptiveMethod),
+                                                       int(thresholdType), blockSize, C))
 
 
 binary_threshold = _thresh("binary")            # utils/color.py:124-137

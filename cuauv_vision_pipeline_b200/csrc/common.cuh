@@ -119,6 +119,8 @@ enum ScratchSlot {
     SCR_HOUGH_ACC,      // int32 Hough accumulators of one group of frames
     SCR_HOUGH_KEYS,     // peak keys of one group of frames, two buffers for the radix sort
     SCR_HOUGH_EDGES,    // edge-pixel lists of one group of frames (+ their values with use_edgeval)
+    SCR_THRESH_SMALL,   // per-frame histograms of the automatic thresholds, or the Gaussian taps of the adaptive one (thresh.cu)
+    SCR_THRESH_PLANE,   // row prefix sums (MEAN_C) or float32 row-filtered frames (GAUSSIAN_C) of the adaptive threshold
     SCR_COUNT
 };
 

@@ -8,6 +8,7 @@
 // 3 x 16 bytes (split planes) with 128-bit stores.  HBM-bound by design: 3 B/px in, 1..6 B/px out.
 #include "common.cuh"
 #include "convert.cuh"
+#include "pointwise.cuh"
 
 namespace bv {
 
@@ -154,25 +155,6 @@ __global__ void __launch_bounds__(256) cvt_inrange_kernel(const uint8_t *__restr
 // ----------------------------------------------------------------------------------------------
 // 1-channel pointwise: inRange, threshold, LUT (16 bytes per thread)
 // ----------------------------------------------------------------------------------------------
-enum Op1 { OP1_INRANGE = 0, OP1_THRESH = 1, OP1_LUT = 2 };
-
-struct Op1Params {
-    int a, b, type;  // inRange: lo, hi;  threshold: thresh, maxval, type
-};
-
-__device__ __forceinline__ uint32_t op1_apply(int op, const Op1Params &p, uint32_t x, const uint8_t *lut) {
-    if (op == OP1_INRANGE) return ((int)x >= p.a && (int)x <= p.b) ? 255u : 0u;
-    if (op == OP1_LUT) return lut[x];
-    const bool above = (int)x > p.a;
-    switch (p.type) {
-        case BV_THRESH_BINARY: return above ? (uint32_t)p.b : 0u;
-        case BV_THRESH_BINARY_INV: return above ? 0u : (uint32_t)p.b;
-        case BV_THRESH_TRUNC: return above ? (uint32_t)p.a : x;
-        case BV_THRESH_TOZERO: return above ? x : 0u;
-        default: return above ? 0u : x;
-    }
-}
-
 template <int OP, bool VEC>
 __global__ void __launch_bounds__(256) op1_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, size_t n,
                                                   Op1Params prm, const uint8_t *__restrict__ g_lut) {

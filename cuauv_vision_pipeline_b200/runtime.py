@@ -231,6 +231,41 @@ class Context:
                                THRESH[kind]))
         return dst
 
+    @staticmethod
+    def _grey_frames(t, what):
+        """(batch, height, width) of a grey frame [H,W] or batch [B,H,W] / [B,H,W,1]."""
+        if t.dim() == 2:
+            return 1, t.shape[0], t.shape[1]
+        if t.dim() == 3 or (t.dim() == 4 and t.shape[3] == 1):
+            return t.shape[0], t.shape[1], t.shape[2]
+        raise BVError(-1, "%s takes [H,W], [B,H,W] or [B,H,W,1]" % what)
+
+    def threshold_auto(self, src, maxval, kind, method):
+        """cv2.threshold(src, 0, maxval, kind | THRESH_OTSU or THRESH_TRIANGLE) of a device frame [H,W] or batch [B,H,W] /
+        [B,H,W,1] (bv_threshold_auto) -> (dst shaped as src, float64 device tensor of the thresholds: [] for a frame,
+        [B] for a batch).  kind: a THRESH name or bv_thresh_type value; method: "otsu" or "triangle"."""
+        self._src(src)
+        b, h, w = self._grey_frames(src, "threshold_auto")
+        dst = self.empty(tuple(src.shape))
+        th = self.empty((b,), torch.float64)
+        check(lib.bv_threshold_auto(self.handle, _u8ptr(src), _u8ptr(dst), b, h, w, float(maxval),
+                                    THRESH[kind] if isinstance(kind, str) else int(kind),
+                                    {"otsu": lib.BV_THRESH_OTSU, "triangle": lib.BV_THRESH_TRIANGLE}[method],
+                                    ffi.cast("double *", th.data_ptr())))
+        return dst, (th[0] if src.dim() == 2 else th)
+
+    def adaptive_threshold(self, src, max_value, method, kind, block_size, c):
+        """cv2.adaptiveThreshold(src, max_value, method, kind, block_size, c) of a device frame [H,W] or batch [B,H,W] /
+        [B,H,W,1] (bv_adaptive_threshold) -> uint8 shaped as src.  method: "mean", "gaussian" or cv2's value; kind:
+        "binary", "binary_inv" or cv2's value.  BVError where cv2 raises."""
+        self._src(src)
+        b, h, w = self._grey_frames(src, "adaptive_threshold")
+        m = {"mean": lib.BV_ADAPTIVE_THRESH_MEAN_C, "gaussian": lib.BV_ADAPTIVE_THRESH_GAUSSIAN_C}.get(method, method)
+        dst = self.empty(tuple(src.shape))
+        check(lib.bv_adaptive_threshold(self.handle, _u8ptr(src), _u8ptr(dst), b, h, w, float(max_value), int(m),
+                                        THRESH[kind] if isinstance(kind, str) else int(kind), int(block_size), float(c)))
+        return dst
+
     def apply_lut(self, src, lut):
         lut = np.ascontiguousarray(lut, dtype=np.uint8)
         channels = 1 if lut.ndim == 1 else lut.shape[0]

@@ -71,6 +71,21 @@ typedef enum bv_thresh_type {
     BV_THRESH_TOZERO_INV = 4  /* x >  t ? 0 : x        */
 } bv_thresh_type;
 
+/* The automatic threshold of bv_threshold_auto (cv2's THRESH_OTSU and THRESH_TRIANGLE flags). */
+typedef enum bv_thresh_auto {
+    BV_THRESH_OTSU = 8,
+    BV_THRESH_TRIANGLE = 16
+} bv_thresh_auto;
+
+/* The local mean of bv_adaptive_threshold (cv2's values). */
+typedef enum bv_adaptive_method {
+    BV_ADAPTIVE_THRESH_MEAN_C = 0,
+    BV_ADAPTIVE_THRESH_GAUSSIAN_C = 1
+} bv_adaptive_method;
+
+/* Largest block_size of bv_adaptive_threshold: the 32-bit window sums of MEAN_C hold 255 * k * k < 2^31. */
+enum { BV_ADAPTIVE_MAX_BLOCK = 2901 };
+
 /* Morphology.  Replaces cv2.erode / cv2.dilate / cv2.morphologyEx as called from
  * utils/transform.py:80-164 and modules/preprocessor.py:120-129. */
 typedef enum bv_morph_op {
@@ -188,6 +203,45 @@ int bv_in_range(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *mask_dev, int batc
 /* cv2.threshold on uint8 (utils/color.py:124-201); n = number of bytes. */
 int bv_threshold(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, size_t n, int thresh, int maxval,
                  int type);
+/* cv2.threshold(src, 0, maxval, type | method) of every frame, method BV_THRESH_OTSU or BV_THRESH_TRIANGLE, matching
+ * OpenCV 4.13.0 bit for bit.  src_dev / dst_dev: uint8 [batch,H,W] (dst_dev == src_dev is allowed: a frame's histogram
+ * is complete before any byte of it is written; any other overlap is BV_ERR_INVALID).  thresh_dev: double [batch], the
+ * threshold cv2 returns for each frame, written on the device (no host synchronisation).  The rules:
+ *   1. Otsu: h = the frame's 256-bin histogram, scale = 1. / (H * W); mu = sum(i * (double)h[i]) * scale; then for
+ *      i = 0..255 in double, every operation rounded on its own (no FMA): p = h[i] * scale; mu1 *= q1; q1 += p;
+ *      q2 = 1 - q1; the bin is skipped when min(q1, q2) < FLT_EPSILON or max(q1, q2) > 1 - FLT_EPSILON;
+ *      mu1 = (mu1 + i * p) / q1; mu2 = (mu - q1 * mu1) / q2; sigma = q1 * q2 * (mu1 - mu2) * (mu1 - mu2); the first
+ *      strict maximum of sigma gives the threshold (0 when no bin qualifies, e.g. a constant frame).
+ *   2. Triangle: left = the first non-empty bin, less one when above 0; right = the last non-empty bin of 1..255 (0 if
+ *      none), plus one when below 255; the peak = the first bin of the largest count.  When peak - left < right - peak
+ *      the histogram is flipped (left = 255 - right, peak = 255 - peak).  Then in float32 with no FMA: a = (float)max,
+ *      b = (float)(left - peak), the first i in left+1..peak with a*i + b*h[i] above every earlier value (starting at
+ *      0, threshold left); the threshold is that i less one, un-flipped (255 - t) when flipped.
+ *   3. the threshold is applied as cv2.threshold applies one on 8-bit: t = floor(thresh), m = cvRound(maxval) (half to
+ *      even; 0 past int32, as on x86-64), m = t for TRUNC, m saturated to 0..255, then the bv_thresh_type rule.
+ * BV_ERR_INVALID (as cv2 raises) for a method other than one of the two, and for a type outside bv_thresh_type; also
+ * for a non-finite maxval, for thresh_dev overlapping src / dst, for frames of 2^31 pixels or more and for batches
+ * above 65535. */
+int bv_threshold_auto(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width,
+                      double maxval, int type, int method, double *thresh_dev);
+/* cv2.adaptiveThreshold(src, max_value, method, type, block_size, c) of every frame, matching OpenCV 4.13.0.
+ * src_dev / dst_dev: uint8 [batch,H,W], not overlapping.  With k = block_size, the local mean m of a pixel is:
+ *   MEAN_C      the integer sum s over the k x k window (BORDER_REPLICATE), as cv2.boxFilter scales it: for k*k <= 2^23
+ *               (k <= 2895) m = cvRound((float)s * (float)(1. / (k*k))), a float32 product (not the exact rounding of
+ *               s / k^2); above (k >= 2897) m = cvRound(s * (1. / (k*k))) in double.  Half to even, bit-exact;
+ *   GAUSSIAN_C  a float32 separable filter of the frame converted to float32, BORDER_REPLICATE, with the taps of
+ *               cv2.getGaussianKernel(k, 0, CV_32F) (built on the host as OpenCV builds them: its dyadic table for
+ *               k <= 9, exp() in double above), rows then columns, each sum taken in tap order, then cvRound to 8 bits.
+ *               Bit-exact for k <= 9 (dyadic taps: every float32 sum is exact); for k >= 11 cv2's own summation order
+ *               depends on its SIMD path, so a pixel may differ where the double-precision mean lies within 1e-3 of a
+ *               half-integer (cv2's own optimised and plain paths disagree at ~1e-4).
+ * then, with d = ceil(c) for BINARY, floor(c) for BINARY_INV and v = saturate_cast<uchar>(max_value) (0 when
+ * max_value < 0): BINARY gives src - m > -d ? v : 0, BINARY_INV gives src - m <= -d ? v : 0.
+ * BV_ERR_INVALID (as cv2 raises) for an even block_size or 1, a method other than the two, a type other than BINARY and
+ * BINARY_INV; also for block_size above BV_ADAPTIVE_MAX_BLOCK, for non-finite max_value or c, for |c| >= 2^31 - 1 (no
+ * int32 for cv2's ceil / floor), for frames of 2^31 pixels or more, and for overlapping src / dst. */
+int bv_adaptive_threshold(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *dst_dev, int batch, int height, int width,
+                          double max_value, int method, int type, int block_size, double c);
 /* cvtColor + inRange in one pass, nothing but the mask is written. */
 int bv_cvt_in_range(bv_ctx *ctx, const uint8_t *src_dev, uint8_t *mask_dev, int batch, int height, int width,
                     int code, const uint8_t *lo_host, const uint8_t *hi_host);
