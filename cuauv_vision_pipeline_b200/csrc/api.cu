@@ -231,9 +231,10 @@ extern "C" int bv_create(int device, bv_ctx **out) {
         return BV_ERR_UNSUPPORTED;
     }
     static const char *const opt_env[BV_OPT_COUNT] = {"BV_HIST_BPS", "BV_FINAL_BPS", "BV_SIDE_STREAMS", "BV_L2_CHUNK_MB",
-                                                      "BV_NO_HUE_TABLE", "BV_CONTOUR_POOL_CHUNKS", "BV_FAST_TABLES", "BV_MORPH_VARIANT", "BV_NO_RCP_TABLES", "BV_FINAL_SV_TABLES", "BV_MORPH_WARPS"};
+                                                      "BV_NO_HUE_TABLE", "BV_CONTOUR_POOL_CHUNKS", nullptr, "BV_MORPH_VARIANT",
+                                                      nullptr, nullptr, "BV_MORPH_WARPS"};   // nullptr: retired option
     for (int i = 0; i < BV_OPT_COUNT; ++i) {
-        const char *v = getenv(opt_env[i]);
+        const char *v = opt_env[i] ? getenv(opt_env[i]) : nullptr;
         ctx->opt[i] = v ? atoi(v) : 0;
     }
     *out = ctx;
@@ -243,6 +244,10 @@ extern "C" int bv_create(int device, bv_ctx **out) {
 extern "C" int bv_set_option(bv_ctx *ctx, int option, int value) {
     BV_REQUIRE(ctx, "null context");
     BV_REQUIRE(option >= 0 && option < BV_OPT_COUNT, "unknown option");
+    if (option == 6 || option == 8 || option == 9) {
+        set_error("bv_set_option: option %d is retired (its alternative implementation was removed)", option);
+        return BV_ERR_INVALID;
+    }
     ctx->opt[option] = value > 0 ? value : 0;
     return BV_OK;
 }

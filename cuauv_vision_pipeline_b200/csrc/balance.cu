@@ -59,7 +59,7 @@ __device__ __forceinline__ int uchar_cast(double v) {
 // channel, sum_i clamp(i, lo, hi) * cnt[i]  (the numerator of cv::mean, 426-428).
 // ----------------------------------------------------------------------------------------------
 // The statistics helpers below are run by the first 256 threads (8 whole warps) of a block, thread t owning bin t; they
-// synchronise on named barrier 1 so that blocks of more than 256 threads (balance_fast.cuh) can call them too.
+// synchronise on named barrier 1 so that blocks of more than 256 threads can call them too.
 __device__ __forceinline__ void stat_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 
 struct StatScratch {
@@ -383,20 +383,16 @@ __device__ __forceinline__ void put_px3(uint32_t (&w)[12], uint32_t (&st)[4], ui
 }
 
 // pixels J..15 of a 16-pixel group of pass 2: tables -> BGR2HSV -> S and V counted, H,S,V packed
-template <int J, bool RCP>
-__device__ __forceinline__ void hsv_group(const Px16 &in, const uint8_t (*lut)[256], const int *sdiv, const int *hdiv,
-                                          uint32_t (*hw)[256], Px16 &o, uint32_t (&stg)[4]) {
+template <int J>
+__device__ __forceinline__ void hsv_group(const Px16 &in, const uint8_t (*lut)[256], uint32_t (*hw)[256], Px16 &o,
+                                          uint32_t (&stg)[4]) {
     if constexpr (J < 16) {
         int hh, ss, vv;
-        if (RCP)
-            bgr2hsv_rcp(lut[0][BV_GETB(in.w, 3 * J)], lut[1][BV_GETB(in.w, 3 * J + 1)], lut[2][BV_GETB(in.w, 3 * J + 2)], hh, ss, vv);
-        else
-            bgr2hsv(lut[0][BV_GETB(in.w, 3 * J)], lut[1][BV_GETB(in.w, 3 * J + 1)], lut[2][BV_GETB(in.w, 3 * J + 2)], sdiv, hdiv, hh,
-                    ss, vv);
+        bgr2hsv_rcp(lut[0][BV_GETB(in.w, 3 * J)], lut[1][BV_GETB(in.w, 3 * J + 1)], lut[2][BV_GETB(in.w, 3 * J + 2)], hh, ss, vv);
         atomicAdd(&hw[0][ss], 1u);
         atomicAdd(&hw[1][vv], 1u);
         put_px3<J>(o.w, stg, (uint32_t)hh, (uint32_t)ss, (uint32_t)vv);
-        hsv_group<J + 1, RCP>(in, lut, sdiv, hdiv, hw, o, stg);
+        hsv_group<J + 1>(in, lut, hw, o, stg);
     }
 }
 
@@ -423,17 +419,14 @@ __device__ __forceinline__ void store_px16_keep(uint8_t *base, size_t group, con
     q[2] = make_uint4(p.w[8], p.w[9], p.w[10], p.w[11]);
 }
 
-}  // namespace bv
-#include "balance_fast.cuh"
-namespace bv {
-
 // ----------------------------------------------------------------------------------------------
 // pass 2: S and V histograms of the table-corrected frame (+ statistics in the last block)
 // ----------------------------------------------------------------------------------------------
 // The full H,S,V of every pixel is kept in `hsv` (frame stride hsv_stride bytes, 16-byte aligned):
-// pass 3 starts from it instead of repeating the three table look-ups and the conversion.
-// RCP: sdiv / hdiv from the reciprocal unit instead of shared memory (pixel_math.cuh: rint_quotient_rcp)
-template <bool VEC, bool RCP>
+// pass 3 starts from it instead of repeating the three table look-ups and the conversion.  Whole 16-pixel groups take
+// sdiv / hdiv from the reciprocal unit instead of shared memory (pixel_math.cuh: rint_quotient_rcp); the scalar tail
+// looks them up.
+template <bool VEC>
 __global__ void __launch_bounds__(kBalThreads) hist_sv_kernel(const uint8_t *__restrict__ src, BalFrame *__restrict__ st,
                                                               size_t npx, uint8_t *__restrict__ hsv, size_t hsv_stride) {
     __shared__ uint32_t h[kBalWarps][2][256];
@@ -461,7 +454,7 @@ __global__ void __launch_bounds__(kBalThreads) hist_sv_kernel(const uint8_t *__r
         if (g + stride < ngroups) load_px16<true>(f, g + stride, nxt);  // prefetch, see pass 1
         Px16 o;
         uint32_t stg[4];
-        hsv_group<0, RCP>(in, lut, sdiv, hdiv, hw, o, stg);
+        hsv_group<0>(in, lut, hw, o, stg);
         store_px16_keep(hf, g, o);
         in = nxt;
     }
@@ -496,72 +489,6 @@ struct FinalSmem {
     int sdiv[256], hdiv[256];
 };
 
-// SVT > 0 (MODE 3, whole 32-pixel groups only): the S / V stretch tables hold what HSV -> BGR starts from instead of the
-// stretched byte.  1: s = S'/255 and v = V'/255 as float32 (the per-pixel int -> float step is gone); 2: 8-byte entries
-// {s, 1 - s} and {v, 2^23 + trunc(v * 255)} (also the max channel and one subtraction).  Same float32 operations in the same
-// order, computed once per table entry instead of once per pixel: results are identical by construction.
-template <int SVT>
-struct SvTabs {
-    float f1[2][256];
-};
-template <>
-struct SvTabs<2> {
-    float2 f2[2][256];
-};
-template <>
-struct SvTabs<0> {};
-
-template <int SVT>
-__device__ __forceinline__ void fill_sv_tabs(SvTabs<SVT> &t, const uint8_t (*lut_sv)[256]) {
-    const float kTwo23 = 8388608.f, inv255 = 1.f / 255.f;
-    if constexpr (SVT > 0) {
-        for (int i = threadIdx.x; i < 512; i += blockDim.x) {
-            const uint32_t n = (&lut_sv[0][0])[i];
-            const float x = __fmaf_rn(__uint_as_float(0x4B000000u | n), inv255, -kTwo23 * inv255);
-            if constexpr (SVT == 1) {
-                (&t.f1[0][0])[i] = x;
-            } else {
-                const float y = i < 256 ? BV_FSUB(1.f, x) : __fadd_rz(BV_FMUL(x, 255.f), kTwo23);
-                (&t.f2[0][0])[i] = make_float2(x, y);
-            }
-        }
-    }
-}
-
-// hsv2bgr_packed<true>(H, S', V', vector path) with S' / V' taken through the tables above (raw S, V index them)
-template <int SVT>
-__device__ __forceinline__ uint32_t hsv2bgr_tab(uint32_t H, uint32_t S, uint32_t V, const SvTabs<SVT> &t) {
-    const float kTwo23 = 8388608.f, hscale = 6.f / 180.f;
-    const float h = __fmaf_rn(__uint_as_float(0x4B000000u | H), hscale, -kTwo23 * hscale);
-    float s, oms, v;
-    uint32_t amax;
-    if constexpr (SVT == 2) {
-        const float2 es = t.f2[0][S], ev = t.f2[1][V];
-        s = es.x;
-        oms = es.y;
-        v = ev.x;
-        amax = __float_as_uint(ev.y);
-    } else {
-        s = t.f1[0][S];
-        v = t.f1[1][V];
-        oms = BV_FSUB(1.f, s);
-        amax = __float_as_uint(__fadd_rz(BV_FMUL(v, 255.f), kTwo23));
-    }
-    const float hfloor = __fadd_rz(h, kTwo23);
-    const int sector = (int)(__float_as_uint(hfloor) & 15u);
-    const float f = BV_FSUB(h, __fsub_rn(hfloor, kTwo23));
-    const float fm = (sector & 1) ? f : BV_FSUB(1.f, f);
-    const float ymin = BV_FMUL(BV_FMUL(v, oms), 255.f);
-    const float ymid = BV_FMUL(BV_FMUL(v, BV_FMA(-s, fm, 1.f)), 255.f);
-    const uint32_t amid = __float_as_uint(__fadd_rz(ymid, kTwo23));
-    const uint32_t amin = __float_as_uint(__fadd_rz(ymin, kTwo23));
-    const uint32_t w = __byte_perm(__byte_perm(amax, amid, 0x2240), amin, 0x3410);
-    const unsigned long long kSel = 0x012ull | (0x102ull << 10) | (0x201ull << 20) | (0x210ull << 30) | (0x120ull << 40) |
-                                    (0x021ull << 50);   // as hsv2bgr_packed (pixel_math.cuh)
-    const uint32_t sel = (uint32_t)(kSel >> (10 * sector)) & 0x3FFu;
-    return __byte_perm(w, 0u, sel | 0x4000u);
-}
-
 // returns the balanced pixel packed as b | g<<8 | r<<16
 template <int MODE>
 __device__ __forceinline__ uint32_t balance_px(uint32_t b, uint32_t g, uint32_t r, bool vec, const FinalSmem &fs) {
@@ -581,18 +508,14 @@ __device__ __forceinline__ uint32_t balance_px(uint32_t b, uint32_t g, uint32_t 
 
 // one group of 16 pixels.  TRACK_X: the group touches the row tail (width % 32 columns), where
 // cv2's scalar HSV2BGR / HLS rounding applies, or wraps to the next row.
-template <int MODE, int CODE, bool TRACK_X, bool NEED_MASK, bool BAL, int SVT, bool CVT, int J>
+template <int MODE, int CODE, bool TRACK_X, bool NEED_MASK, bool BAL, bool CVT, int J>
 struct GroupBody {
     static __device__ __forceinline__ void run(const Px16 &in, int x, int width, int vec_end, const FinalSmem &fs,
-                                               const SvTabs<SVT> &svt, const SmemTabs &tabs, const RangeTest &bd, Px16 &ob,
-                                               Px16 &oc, uint32_t (&q)[4], uint32_t &bits, uint32_t (&stg)[4]) {
+                                               const SmemTabs &tabs, const RangeTest &bd, Px16 &ob, Px16 &oc, uint32_t (&q)[4],
+                                               uint32_t &bits, uint32_t (&stg)[4]) {
         constexpr bool kOne = CvtTraits<CODE>::kOneChannel;
         const bool vec = TRACK_X ? (x < vec_end) : true;
-        uint32_t p;
-        if constexpr (SVT > 0 && MODE == 3 && !TRACK_X)
-            p = hsv2bgr_tab<SVT>(BV_GETB(in.w, 3 * J), BV_GETB(in.w, 3 * J + 1), BV_GETB(in.w, 3 * J + 2), svt);
-        else
-            p = balance_px<MODE>(BV_GETB(in.w, 3 * J), BV_GETB(in.w, 3 * J + 1), BV_GETB(in.w, 3 * J + 2), vec, fs);
+        const uint32_t p = balance_px<MODE>(BV_GETB(in.w, 3 * J), BV_GETB(in.w, 3 * J + 1), BV_GETB(in.w, 3 * J + 2), vec, fs);
         if (BAL) put_px<J>(ob.w, p);   // packing the balanced pixel costs ~2.5 instructions: only when that output exists
         int o0, o1, o2;
         convert_px<CODE>((int)(p & 0xFF), (int)((p >> 8) & 0xFF), (int)(p >> 16), vec, tabs, o0, o1, o2);
@@ -608,25 +531,23 @@ struct GroupBody {
         if (TRACK_X) {
             if (++x == width) x = 0;
         }
-        GroupBody<MODE, CODE, TRACK_X, NEED_MASK, BAL, SVT, CVT, J + 1>::run(in, x, width, vec_end, fs, svt, tabs, bd, ob, oc, q, bits, stg);
+        GroupBody<MODE, CODE, TRACK_X, NEED_MASK, BAL, CVT, J + 1>::run(in, x, width, vec_end, fs, tabs, bd, ob, oc, q, bits, stg);
     }
 };
-template <int MODE, int CODE, bool TRACK_X, bool NEED_MASK, bool BAL, int SVT, bool CVT>
-struct GroupBody<MODE, CODE, TRACK_X, NEED_MASK, BAL, SVT, CVT, 16> {
-    static __device__ __forceinline__ void run(const Px16 &, int, int, int, const FinalSmem &, const SvTabs<SVT> &,
-                                               const SmemTabs &, const RangeTest &, Px16 &, Px16 &, uint32_t (&)[4], uint32_t &,
-                                               uint32_t (&)[4]) {}
+template <int MODE, int CODE, bool TRACK_X, bool NEED_MASK, bool BAL, bool CVT>
+struct GroupBody<MODE, CODE, TRACK_X, NEED_MASK, BAL, CVT, 16> {
+    static __device__ __forceinline__ void run(const Px16 &, int, int, int, const FinalSmem &, const SmemTabs &, const RangeTest &,
+                                               Px16 &, Px16 &, uint32_t (&)[4], uint32_t &, uint32_t (&)[4]) {}
 };
 
 // BAL: the balanced image is an output (always when CODE == -1); without it the vector path skips packing it
-template <int MODE, int CODE, bool VEC, bool NEED_MASK, bool BAL = true, int SVT = 0, bool CVT = true>
+template <int MODE, int CODE, bool VEC, bool NEED_MASK, bool BAL = true, bool CVT = true>
 __global__ void __launch_bounds__(kBalThreads) final_kernel(const uint8_t *__restrict__ src, size_t src_stride,
                                                             const BalFrame *__restrict__ st, size_t npx, int width,
                                                             BalOutputs out, const uint16_t *__restrict__ g_gamma,
                                                             const uint16_t *__restrict__ g_cbrt) {
     __shared__ FinalSmem fs;
     __shared__ SmemTabs tabs;
-    __shared__ SvTabs<SVT> svt;
     const int frame = blockIdx.y;
     if (MODE == 2) {
         for (int i = threadIdx.x; i < 256; i += blockDim.x) {
@@ -640,7 +561,6 @@ __global__ void __launch_bounds__(kBalThreads) final_kernel(const uint8_t *__res
         for (int i = threadIdx.x; i < 768; i += blockDim.x) (&fs.lut[0][0])[i] = (&st[frame].lut_bgr[0][0])[i];
     if (MODE >= 2)
         for (int i = threadIdx.x; i < 512; i += blockDim.x) (&fs.lut_sv[0][0])[i] = (&st[frame].lut_sv[0][0])[i];
-    fill_sv_tabs<SVT>(svt, st[frame].lut_sv);
     __syncthreads();
     const size_t foff = (size_t)frame * npx;
     const uint8_t *f = src + (size_t)frame * src_stride;  // BGR frame, or pass 2's H,S,V scratch (MODE 3)
@@ -668,9 +588,9 @@ __global__ void __launch_bounds__(kBalThreads) final_kernel(const uint8_t *__res
 #pragma unroll
         for (int k = 0; k < 12; ++k) ob.w[k] = oc.w[k] = 0;
         if (kNeedX && (int)x0 + 16 > vec_end)
-            GroupBody<MODE, CODE, true, NEED_MASK, BAL, SVT, CVT, 0>::run(in, (int)x0, width, vec_end, fs, svt, tabs, bd, ob, oc, q, bits, stg);
+            GroupBody<MODE, CODE, true, NEED_MASK, BAL, CVT, 0>::run(in, (int)x0, width, vec_end, fs, tabs, bd, ob, oc, q, bits, stg);
         else
-            GroupBody<MODE, CODE, false, NEED_MASK, BAL, SVT, CVT, 0>::run(in, (int)x0, width, vec_end, fs, svt, tabs, bd, ob, oc, q, bits, stg);
+            GroupBody<MODE, CODE, false, NEED_MASK, BAL, CVT, 0>::run(in, (int)x0, width, vec_end, fs, tabs, bd, ob, oc, q, bits, stg);
         if (BAL && out.balanced) store_px16(out.balanced + foff * 3, g, ob);
         if (CVT && out.converted) {
             if (kOne)
@@ -1188,11 +1108,6 @@ static int balance_run_tiled(bv_ctx *ctx, const uint8_t *src, int batch, int hei
 // lone chunk (single frame, or profiling) gets the whole machine.
 static int hist_blocks_per_sm(const bv_ctx *ctx) { return ctx->opt[BV_OPT_HIST_BPS] > 0 ? ctx->opt[BV_OPT_HIST_BPS] : (ctx->overlapped ? 2 : 4); }
 static int final_blocks_per_sm(const bv_ctx *ctx) { return ctx->opt[BV_OPT_FINAL_BPS] > 0 ? ctx->opt[BV_OPT_FINAL_BPS] : (ctx->overlapped ? 2 : 8); }
-static int side_streams(const bv_ctx *ctx) {
-    const int v = ctx->opt[BV_OPT_SIDE_STREAMS] > 0 ? ctx->opt[BV_OPT_SIDE_STREAMS] : 4;
-    return v > BV_MAX_SIDE ? BV_MAX_SIDE : v;
-}
-static size_t l2_chunk_bytes(const bv_ctx *ctx) { return (size_t)(ctx->opt[BV_OPT_L2_CHUNK_MB] > 0 ? ctx->opt[BV_OPT_L2_CHUNK_MB] : 33) << 20; }
 
 static bool vec_ok(const void *p, size_t npx, int batch, int bytes_per_px) {
     (void)bytes_per_px;
@@ -1213,16 +1128,8 @@ static int launch_final(bv_ctx *ctx, const uint8_t *src, size_t src_stride, cons
 #define BV_FINAL_NOBAL(M)                                                                                                     \
     BV_LAUNCH_PDL(ctx, (final_kernel<MODE, CODE, true, M, false>), grid, kBalThreads, 0, src, src_stride, st, npx, width, out, \
                   ctx->d_lab_gamma, ctx->d_lab_cbrt)
-    const int svt = ctx->opt[BV_OPT_FINAL_SV_TABLES];
-    if (MODE == 3 && CODE == BV_BGR2LAB && vec && !out.balanced && !need_mask && svt > 0) {   // experiment: DESIGN.md 4b
-        if (svt == 1)
-            BV_LAUNCH_PDL(ctx, (final_kernel<MODE, CODE, true, false, false, (MODE == 3 && CODE == BV_BGR2LAB) ? 1 : 0>), grid,
-                          kBalThreads, 0, src, src_stride, st, npx, width, out, ctx->d_lab_gamma, ctx->d_lab_cbrt);
-        else
-            BV_LAUNCH_PDL(ctx, (final_kernel<MODE, CODE, true, false, false, (MODE == 3 && CODE == BV_BGR2LAB) ? 2 : 0>), grid,
-                          kBalThreads, 0, src, src_stride, st, npx, width, out, ctx->d_lab_gamma, ctx->d_lab_cbrt);
-    } else if (vec && CODE != -1 && !out.balanced && !out.converted && need_mask) {   // mask only (modules/bins.py, red_buoy.py)
-        BV_LAUNCH_PDL(ctx, (final_kernel<MODE, CODE, true, true, false, 0, false>), grid, kBalThreads, 0, src, src_stride, st, npx,
+    if (vec && CODE != -1 && !out.balanced && !out.converted && need_mask) {   // mask only (modules/bins.py, red_buoy.py)
+        BV_LAUNCH_PDL(ctx, (final_kernel<MODE, CODE, true, true, false, false>), grid, kBalThreads, 0, src, src_stride, st, npx,
                       width, out, ctx->d_lab_gamma, ctx->d_lab_cbrt);
     } else if (vec && CODE != -1 && !out.balanced) {   // the common module case: only the converted image / the mask leave the pass
         if (need_mask) BV_FINAL_NOBAL(true); else BV_FINAL_NOBAL(false);
@@ -1255,8 +1162,6 @@ static bool all_vec(const uint8_t *src, const BalOutputs &out, size_t npx, int b
            vec_ok(out.mask, npx, batch, 1);
 }
 
-static int rcp_tables_usable(bv_ctx *ctx, bool *ok);
-
 // sdiv / hdiv through the reciprocal unit: compared once per context with the integer formulas, all 2 x 256 values
 __global__ void rcp_tables_check_kernel(int *bad) {
     const int d = threadIdx.x;
@@ -1266,80 +1171,17 @@ __global__ void rcp_tables_check_kernel(int *bad) {
 }
 
 int rcp_tables_check(bv_ctx *ctx) {   // called by bv_create: every BGR2HSV of the library relies on it
-    bool ok = false;
-    BV_TRY(rcp_tables_usable(ctx, &ok));
-    if (ctx->rcp_state != 1) {
+    if (!ctx->d_ivl_flag) BV_CUDA(cudaMalloc(&ctx->d_ivl_flag, sizeof(int)));
+    BV_CUDA(cudaMemsetAsync(ctx->d_ivl_flag, 0, sizeof(int), ctx->stream));
+    BV_LAUNCH(ctx, rcp_tables_check_kernel, 1, 256, 0, ctx->d_ivl_flag);
+    int bad = 1;
+    BV_CUDA(cudaMemcpyAsync(&bad, ctx->d_ivl_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    BV_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (bad) {
         set_error("bv_create: rcp.approx.f32 of this device does not reproduce OpenCV's sdiv / hdiv tables (library is built for sm_100a)");
         return BV_ERR_UNSUPPORTED;
     }
     return BV_OK;
-}
-
-static int rcp_tables_usable(bv_ctx *ctx, bool *ok) {
-    if (ctx->rcp_state == 0) {
-        if (!ctx->d_ivl_flag) BV_CUDA(cudaMalloc(&ctx->d_ivl_flag, sizeof(int)));
-        BV_CUDA(cudaMemsetAsync(ctx->d_ivl_flag, 0, sizeof(int), ctx->stream));
-        BV_LAUNCH(ctx, rcp_tables_check_kernel, 1, 256, 0, ctx->d_ivl_flag);
-        int bad = 1;
-        BV_CUDA(cudaMemcpyAsync(&bad, ctx->d_ivl_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-        BV_CUDA(cudaStreamSynchronize(ctx->stream));
-        ctx->rcp_state = bad ? 2 : 1;
-    }
-    *ok = ctx->rcp_state == 1 && ctx->opt[BV_OPT_NO_RCP_TABLES] <= 0;
-    return BV_OK;
-}
-
-// ---- fast passes 2 and 3 (balance_fast.cuh): 512-thread blocks, two per SM, ~107 KB of replicated tables each ----
-static int fast_blocks_per_frame(const bv_ctx *ctx, int nf, size_t npx) {
-    int bpf = (ctx->sm_count * 2 + nf - 1) / nf;
-    const size_t need = (npx / 16 + kFastThreads - 1) / kFastThreads;
-    if ((size_t)bpf > need) bpf = (int)(need ? need : 1);
-    return bpf;
-}
-
-template <typename K>
-static int enable_fast_smem(bv_ctx *ctx, K kernel, int bit, size_t bytes) {
-    if (!(ctx->fast_attr_set & (1u << bit))) {  // per context, hence per device
-        BV_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        ctx->fast_attr_set |= 1u << bit;
-    }
-    return BV_OK;
-}
-
-static int launch_hist_sv_fast(bv_ctx *ctx, const uint8_t *src, BalFrame *st, int nf, size_t npx, uint8_t *hsv, size_t hsv_stride) {
-    BV_TRY(enable_fast_smem(ctx, hist_sv_fast_kernel, 0, sizeof(Sv2Smem)));
-    dim3 grid(fast_blocks_per_frame(ctx, nf, npx), nf);
-    BV_LAUNCH_PDL(ctx, hist_sv_fast_kernel, grid, kFastThreads, sizeof(Sv2Smem), src, st, npx, hsv, hsv_stride);
-    return BV_OK;
-}
-
-template <int CODE, int BIT>
-static int launch_final_fast(bv_ctx *ctx, const uint8_t *hsv, size_t hsv_stride, const BalFrame *st, int nf, size_t npx, int width,
-                             const BalOutputs &out) {
-    const size_t smem = CODE == BV_BGR2LAB ? sizeof(Fin2Smem) : sizeof(Fin2SmemSmall);
-    dim3 grid(fast_blocks_per_frame(ctx, nf, npx), nf);
-    if (out.mask || out.mask_bits) {
-        BV_TRY(enable_fast_smem(ctx, final_fast_kernel<CODE, true>, BIT, smem));
-        BV_LAUNCH_PDL(ctx, (final_fast_kernel<CODE, true>), grid, kFastThreads, smem, hsv, hsv_stride, st, npx, width, out,
-                      ctx->d_lab_gamma, ctx->d_lab_cbrt);
-    } else {
-        BV_TRY(enable_fast_smem(ctx, final_fast_kernel<CODE, false>, BIT + 1, smem));
-        BV_LAUNCH_PDL(ctx, (final_fast_kernel<CODE, false>), grid, kFastThreads, smem, hsv, hsv_stride, st, npx, width, out,
-                      ctx->d_lab_gamma, ctx->d_lab_cbrt);
-    }
-    return BV_OK;
-}
-
-static int dispatch_final_fast(bv_ctx *ctx, const uint8_t *hsv, size_t hsv_stride, const BalFrame *st, int nf, size_t npx, int width,
-                               int code, const BalOutputs &out) {
-    switch (code) {
-        case -1: return launch_final_fast<-1, 1>(ctx, hsv, hsv_stride, st, nf, npx, width, out);
-        case BV_BGR2HSV: return launch_final_fast<BV_BGR2HSV, 3>(ctx, hsv, hsv_stride, st, nf, npx, width, out);
-        case BV_BGR2LAB: return launch_final_fast<BV_BGR2LAB, 5>(ctx, hsv, hsv_stride, st, nf, npx, width, out);
-        case BV_BGR2GRAY: return launch_final_fast<BV_BGR2GRAY, 7>(ctx, hsv, hsv_stride, st, nf, npx, width, out);
-        case BV_BGR2YCRCB: return launch_final_fast<BV_BGR2YCRCB, 9>(ctx, hsv, hsv_stride, st, nf, npx, width, out);
-        default: return 1;  // not covered: the caller takes the generic pass
-    }
 }
 
 int convert_run(bv_ctx *ctx, const uint8_t *src, int batch, int height, int width, int cvt_code, const BalOutputs &out) {
@@ -1421,11 +1263,6 @@ int balance_run(bv_ctx *ctx, const uint8_t *src, int batch, int height, int widt
         }
     }
 
-    bool rcp = false;
-    if (prm.hsv_contrast_correct) BV_TRY(rcp_tables_usable(ctx, &rcp));
-    // conflict-free tables (balance_fast.cuh): whole 16-pixel groups, aligned buffers
-    const bool fast = prm.hsv_contrast_correct && vec && npx % 16 == 0 && ctx->opt[BV_OPT_FAST_TABLES] > 0;
-
     // chunk the batch so that one chunk's input stays in L2 across the three passes; chunks are
     // independent and alternate over side streams so that their passes overlap on the SMs
     int chunk = (int)(l2_chunk_bytes(ctx) / (npx * 3));
@@ -1445,25 +1282,7 @@ int balance_run(bv_ctx *ctx, const uint8_t *src, int batch, int height, int widt
     if (ctx->opt[BV_OPT_L2_CHUNK_MB] <= 0 && (size_t)(2 * chunk) * npx * 3 <= ((size_t)80 << 20) &&
         batch >= 2 * chunk * side_streams(ctx))
         chunk *= 2;
-    if (chunk < 1) chunk = 1;
-    const int nchunks = (batch + chunk - 1) / chunk;
-    int nside = side_streams(ctx);
-    if (nside > nchunks) nside = nchunks;
-    if (ctx->prof) nside = 1;  // per-kernel timing wants serialised launches
-    cudaStream_t main_stream = ctx->stream;
-    ctx->overlapped = nside > 1;
-    if (nside > 1) {
-        BV_CUDA(cudaEventRecord(ctx->ev_fork, main_stream));
-        for (int i = 0; i < nside; ++i) BV_CUDA(cudaStreamWaitEvent(ctx->side[i], ctx->ev_fork, 0));
-    }
-    struct Restore {  // every exit path puts the context's stream back
-        bv_ctx *c;
-        cudaStream_t s;
-        ~Restore() { c->stream = s; }
-    } restore{ctx, main_stream};
-    for (int f0 = 0, ci = 0; f0 < batch; f0 += chunk, ++ci) {
-        if (nside > 1) ctx->stream = ctx->side[ci % nside];
-        const int nf = batch - f0 < chunk ? batch - f0 : chunk;
+    BV_TRY(for_chunks_on_side_streams(ctx, batch, chunk, [&](int f0, int nf) -> int {
         const uint8_t *csrc = src + (size_t)f0 * npx * 3;
         BalFrame *cst = st + f0;
         uint8_t *chsv = hsv ? hsv + (size_t)f0 * hsv_stride : nullptr;
@@ -1476,40 +1295,25 @@ int balance_run(bv_ctx *ctx, const uint8_t *src, int batch, int height, int widt
         else
             BV_LAUNCH(ctx, hist_bgr_kernel<false>, grid, kBalThreads, 0, csrc, cst, npx, prm, ctx->d_pow_quarter);
         if (prm.hsv_contrast_correct) {
-            if (fast)
-                BV_TRY(launch_hist_sv_fast(ctx, csrc, cst, nf, npx, chsv, hsv_stride));
-            else if (vec && rcp)
-                BV_LAUNCH_PDL(ctx, (hist_sv_kernel<true, true>), grid, kBalThreads, 0, csrc, cst, npx, chsv, hsv_stride);
-            else if (vec)
-                BV_LAUNCH_PDL(ctx, (hist_sv_kernel<true, false>), grid, kBalThreads, 0, csrc, cst, npx, chsv, hsv_stride);
+            if (vec)
+                BV_LAUNCH_PDL(ctx, hist_sv_kernel<true>, grid, kBalThreads, 0, csrc, cst, npx, chsv, hsv_stride);
             else
-                BV_LAUNCH_PDL(ctx, (hist_sv_kernel<false, false>), grid, kBalThreads, 0, csrc, cst, npx, chsv, hsv_stride);
+                BV_LAUNCH_PDL(ctx, hist_sv_kernel<false>, grid, kBalThreads, 0, csrc, cst, npx, chsv, hsv_stride);
         }
         BalOutputs co = out;
         if (co.balanced) co.balanced += (size_t)f0 * npx * 3;
         if (co.converted) co.converted += (size_t)f0 * npx * (cvt_code == BV_BGR2GRAY ? 1 : 3);
         if (co.mask) co.mask += (size_t)f0 * npx;
         if (co.mask_bits) co.mask_bits += (size_t)f0 * height * (((width + 31) / 32) * 2);
-        if (ivl) {
+        if (ivl)
             BV_TRY(launch_mask_from_hsv(ctx, chsv, hsv_stride, cst, nf, npx, width, ivl, ivl_frames + (size_t)f0 * kIvlEntries, co));
-        } else if (prm.hsv_contrast_correct) {
-            int s3 = 1;  // 1: the fast pass does not cover this case
-            if (fast && width % 32 == 0) {
-                s3 = dispatch_final_fast(ctx, chsv, hsv_stride, cst, nf, npx, width, cvt_code, co);
-                if (s3 < 0) return s3;
-            }
-            if (s3 == 1) BV_TRY(dispatch_final<3>(ctx, chsv, hsv_stride, cst, nf, npx, width, cvt_code, co, vec));
-        }
+        else if (prm.hsv_contrast_correct)
+            BV_TRY(dispatch_final<3>(ctx, chsv, hsv_stride, cst, nf, npx, width, cvt_code, co, vec));
         else
             BV_TRY(dispatch_final<1>(ctx, csrc, npx * 3, cst, nf, npx, width, cvt_code, co, vec));
         if (after_chunk) BV_TRY(after_chunk->fn(after_chunk->self, ctx, f0, nf));
-    }
-    ctx->stream = main_stream;
-    if (nside > 1)
-        for (int i = 0; i < nside; ++i) {
-            BV_CUDA(cudaEventRecord(ctx->ev_join[i], ctx->side[i]));
-            BV_CUDA(cudaStreamWaitEvent(main_stream, ctx->ev_join[i], 0));
-        }
+        return BV_OK;
+    }));
     if (stats_host) {
         BV_CUDA(cudaMemcpy2DAsync(stats_host, sizeof(bv_balance_stats), &st[0].stats, sizeof(BalFrame),
                                   sizeof(bv_balance_stats), batch, cudaMemcpyDeviceToHost, ctx->stream));

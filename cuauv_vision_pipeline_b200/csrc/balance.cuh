@@ -1,8 +1,51 @@
-// balance.cuh -- device-side state of the colour balance, shared by balance.cu and stage.cu.
+// balance.cuh -- device-side state of the colour balance and the chunking policy of a batch, shared by balance.cu and
+// stage.cu.
 #pragma once
 #include "common.cuh"
 
 namespace bv {
+
+// Chunking of a batch (bv_set_option / BV_* environment variables read at bv_create, see api.cu): independent chunks in
+// flight on side streams, and the input bytes per chunk that keep a chunk and its H,S,V scratch in L2 across the passes.
+inline int side_streams(const bv_ctx *ctx) {
+    const int v = ctx->opt[BV_OPT_SIDE_STREAMS] > 0 ? ctx->opt[BV_OPT_SIDE_STREAMS] : 4;
+    return v > BV_MAX_SIDE ? BV_MAX_SIDE : v;
+}
+inline size_t l2_chunk_bytes(const bv_ctx *ctx) { return (size_t)(ctx->opt[BV_OPT_L2_CHUNK_MB] > 0 ? ctx->opt[BV_OPT_L2_CHUNK_MB] : 33) << 20; }
+
+// Runs fn(f0, nf) for consecutive chunks of the batch, alternating over the side streams (fork from / join into the
+// context's stream).  ctx->overlapped tells the kernels' grid sizing whether chunks share the SMs.
+template <class Fn>
+int for_chunks_on_side_streams(bv_ctx *ctx, int batch, int chunk, Fn fn) {
+    if (chunk < 1) chunk = 1;
+    const int nchunks = (batch + chunk - 1) / chunk;
+    int nside = side_streams(ctx);
+    if (nside > nchunks) nside = nchunks;
+    if (ctx->prof) nside = 1;  // per-kernel timing wants serialised launches
+    cudaStream_t main_stream = ctx->stream;
+    ctx->overlapped = nside > 1;
+    if (nside > 1) {
+        BV_CUDA(cudaEventRecord(ctx->ev_fork, main_stream));
+        for (int i = 0; i < nside; ++i) BV_CUDA(cudaStreamWaitEvent(ctx->side[i], ctx->ev_fork, 0));
+    }
+    struct Restore {  // every exit path puts the context's stream back
+        bv_ctx *c;
+        cudaStream_t s;
+        ~Restore() { c->stream = s; }
+    } restore{ctx, main_stream};
+    for (int k = 0; k < nchunks; ++k) {
+        const int f0 = k * chunk, nf = (batch - f0 < chunk) ? batch - f0 : chunk;
+        if (nside > 1) ctx->stream = ctx->side[k % nside];
+        BV_TRY(fn(f0, nf));
+    }
+    ctx->stream = main_stream;
+    if (nside > 1)
+        for (int i = 0; i < nside; ++i) {
+            BV_CUDA(cudaEventRecord(ctx->ev_join[i], ctx->side[i]));
+            BV_CUDA(cudaStreamWaitEvent(main_stream, ctx->ev_join[i], 0));
+        }
+    return BV_OK;
+}
 
 // Per-frame working state in HBM (3.9 KB + 1.75 KB of tables per tile).
 struct BalFrame {

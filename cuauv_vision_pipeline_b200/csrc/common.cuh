@@ -163,8 +163,6 @@ struct bv_ctx {
     } ivl[BV_IVL_SLOTS];
     int ivl_next;
     int ivl_attr_set;
-    int rcp_state;           // sdiv / hdiv through the reciprocal unit: 0 not checked yet, 1 identical to the tables on this device, 2 not
-    unsigned fast_attr_set;  // bit per instantiation of the fast passes whose dynamic shared-memory size has been enabled
     int lb_smem_set;     // same for letterbox_tma_kernel
     void *lb_cache;      // host copy of the letterbox descriptors whose tap table is on the device
     int lb_cache_n, lb_cache_ow, lb_cache_oh;

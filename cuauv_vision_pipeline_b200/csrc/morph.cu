@@ -284,11 +284,6 @@ __device__ __forceinline__ void chain_step(uint32_t *A, uint32_t *B, int rows, i
     __syncthreads();
 }
 
-// TMA: the tile's rows are one contiguous byte range of the frame; when it starts and ends on 16 bytes one thread hands
-// it to the TMA engine as a single bulk copy (cp.async.bulk, SASS UBLKCP) completing on an mbarrier, rows outside the
-// image are zero-filled by the block.  (Tensor-map TMA with out-of-bounds fill needs a 16-byte row pitch; a bit-packed
-// 2208-px row is 276 bytes.)
-template <bool TMA>
 __global__ void __launch_bounds__(kChainThreads) morph_chain_kernel(const uint32_t *__restrict__ src,
                                                                     uint32_t *__restrict__ dst_bits, uint8_t *__restrict__ mask,
                                                                     int height, int width, int wpr, int tiles_per_frame,
@@ -300,37 +295,10 @@ __global__ void __launch_bounds__(kChainThreads) morph_chain_kernel(const uint32
     uint32_t *A = chain_smem, *B = chain_smem + rows * wpr;
     const uint32_t *fsrc = src + (size_t)frame * height * wpr;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    bool staged = false;
-    if (TMA) {
-        __shared__ uint64_t bar;
-        const int ya = max(ybase, 0), yb = min(ybase + rows, height);           // rows of the tile inside the image
-        const size_t off = (size_t)ya * wpr * 4, bytes = (size_t)(yb - ya) * wpr * 4;
-        const uint32_t *g = fsrc + (size_t)ya * wpr;
-        uint32_t *d = A + (ya - ybase) * wpr;
-        // uniform for the block: source, destination and size on 16 bytes
-        if (yb > ya && ((reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(d) | bytes) & 15) == 0) {
-            (void)off;
-            if (threadIdx.x == 0) {
-                mbar_init(&bar, 1);
-                mbar_expect_tx(&bar, (uint32_t)bytes);
-                bulk_g2s(d, g, (uint32_t)bytes, &bar);
-            }
-            for (int r = warp; r < rows; r += nwarps) {
-                const int y = ybase + r;
-                if (y < 0 || y >= height)
-                    for (int wx = lane; wx < wpr; wx += 32) A[r * wpr + wx] = 0u;
-            }
-            __syncthreads();
-            mbar_wait(&bar, 0);
-            staged = true;
-        }
-    }
-    if (!staged) {
-        for (int r = warp; r < rows; r += nwarps) {
-            const int y = ybase + r;
-            const bool inside = y >= 0 && y < height;
-            for (int wx = lane; wx < wpr; wx += 32) A[r * wpr + wx] = inside ? __ldg(fsrc + (size_t)y * wpr + wx) : 0u;
-        }
+    for (int r = warp; r < rows; r += nwarps) {
+        const int y = ybase + r;
+        const bool inside = y >= 0 && y < height;
+        for (int wx = lane; wx < wpr; wx += 32) A[r * wpr + wx] = inside ? __ldg(fsrc + (size_t)y * wpr + wx) : 0u;
     }
     __syncthreads();
     const int last = wpr - 1;
@@ -575,18 +543,13 @@ int morph_bits_chain(bv_ctx *ctx, const uint32_t *bits, uint32_t *dst_bits, uint
         std::lock_guard<std::mutex> lock(mu);
         int &cur = enabled[ctx->device];
         if ((int)smem > cur) {
-            BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            BV_CUDA(cudaFuncSetAttribute(morph_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             cur = (int)smem;
         }
     }
     const int tiles = (height + tile_rows - 1) / tile_rows;
-    if (ctx->opt[BV_OPT_MORPH_VARIANT] == 2)
-        BV_LAUNCH(ctx, morph_chain_kernel<true>, batch * tiles, kChainThreads, smem, bits, dst_bits, mask, height, width, wpr, tiles,
-                  tile_rows, ch);
-    else
-        BV_LAUNCH(ctx, morph_chain_kernel<false>, batch * tiles, kChainThreads, smem, bits, dst_bits, mask, height, width, wpr, tiles,
-                  tile_rows, ch);
+    BV_LAUNCH(ctx, morph_chain_kernel, batch * tiles, kChainThreads, smem, bits, dst_bits, mask, height, width, wpr, tiles,
+              tile_rows, ch);
     *done = true;
     return BV_OK;
 }

@@ -75,7 +75,7 @@ BV_HD void bgr2hsv(int b, int g, int r, const int *sdiv, const int *hdiv, int &h
 // 1 / (2d) away from the nearest rounding boundary, while the computed value is off by at most
 // num / d * (2^-23 [rcp.approx, 1 ulp] + 2^-24 [the multiply]) <= 0.19 / d.  d = 0 gives 1 / 0 = +inf, whose sum with the
 // magic constant keeps an all-zero low mantissa: 0, as the tables define.  rcp_tables_check_kernel (balance.cu) compares
-// all 2 x 256 values with the integer formulas on the device once per context; a mismatch switches the tables back on.
+// all 2 x 256 values with the integer formulas on the device when a context is created; bv_create fails on a mismatch.
 __device__ __forceinline__ int rint_quotient_rcp(float num, int d) {
     const float df = __fsub_rn(__uint_as_float(0x4B000000u | (uint32_t)d), 8388608.f);   // float(d) without the conversion unit
     float r;

@@ -81,40 +81,6 @@ struct StageTail {
     static int hook(void *self, bv_ctx *c, int f0, int nf) { return ((StageTail *)self)->run(c, f0, nf); }
 };
 
-// Runs fn(f0, nf) for consecutive chunks of the batch, alternating over the side streams (fork from / join into the
-// context's stream), like balance_run does for its own chunks.
-template <class Fn>
-static int for_chunks_on_side_streams(bv_ctx *ctx, int batch, int chunk, Fn fn) {
-    if (chunk < 1) chunk = 1;
-    const int nchunks = (batch + chunk - 1) / chunk;
-    int nside = ctx->opt[BV_OPT_SIDE_STREAMS] > 0 ? ctx->opt[BV_OPT_SIDE_STREAMS] : 4;
-    if (nside > BV_MAX_SIDE) nside = BV_MAX_SIDE;
-    if (nside > nchunks) nside = nchunks;
-    if (ctx->prof) nside = 1;  // per-kernel timing wants serialised launches
-    cudaStream_t main_stream = ctx->stream;
-    if (nside > 1) {
-        BV_CUDA(cudaEventRecord(ctx->ev_fork, main_stream));
-        for (int i = 0; i < nside; ++i) BV_CUDA(cudaStreamWaitEvent(ctx->side[i], ctx->ev_fork, 0));
-    }
-    struct Restore {  // every exit path puts the context's stream back
-        bv_ctx *c;
-        cudaStream_t s;
-        ~Restore() { c->stream = s; }
-    } restore{ctx, main_stream};
-    for (int k = 0; k < nchunks; ++k) {
-        const int f0 = k * chunk, nf = (batch - f0 < chunk) ? batch - f0 : chunk;
-        if (nside > 1) ctx->stream = ctx->side[k % nside];
-        BV_TRY(fn(f0, nf));
-    }
-    ctx->stream = main_stream;
-    if (nside > 1)
-        for (int i = 0; i < nside; ++i) {
-            BV_CUDA(cudaEventRecord(ctx->ev_join[i], ctx->side[i]));
-            BV_CUDA(cudaStreamWaitEvent(main_stream, ctx->ev_join[i], 0));
-        }
-    return BV_OK;
-}
-
 int stage_run(bv_ctx *ctx, const bv_stage_desc *desc, const uint8_t *src, int batch, int height, int width,
               uint8_t *balanced, uint8_t *converted, uint8_t *mask, int32_t *labels, bv_blob *blobs, int max_blobs,
               int32_t *n_blobs) {
@@ -184,8 +150,7 @@ int stage_run(bv_ctx *ctx, const bv_stage_desc *desc, const uint8_t *src, int ba
     // when the work is worth splitting
     int chunk = batch;
     if (need_bits && batch > 1) {
-        const size_t l2_chunk = (size_t)(ctx->opt[BV_OPT_L2_CHUNK_MB] > 0 ? ctx->opt[BV_OPT_L2_CHUNK_MB] : 33) << 20;
-        chunk = (int)(l2_chunk / (npx * 3));
+        chunk = (int)(l2_chunk_bytes(ctx) / (npx * 3));
         const int quarter = (batch + 3) / 4;
         if (chunk > quarter) chunk = quarter;
         const size_t min_px = (size_t)1 << 20;   // below ~1 Mpx per chunk the launches cost more than the overlap returns

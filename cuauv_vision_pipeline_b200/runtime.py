@@ -92,7 +92,7 @@ class Context:
         return int(lib.bv_launch_count(self.handle))
 
     OPTIONS = {"hist_bps": 0, "final_bps": 1, "side_streams": 2, "l2_chunk_mb": 3, "no_hue_table": 4, "contour_pool_chunks": 5,
-               "fast_tables": 6, "morph_variant": 7, "no_rcp_tables": 8, "final_sv_tables": 9, "morph_warps": 10}
+               "morph_variant": 7, "morph_warps": 10}
 
     def set_option(self, name, value):
         """Tuning knob of the colour-balance passes (include/b200vision.h, BV_OPT_*); 0 = default."""

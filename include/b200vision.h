@@ -169,11 +169,8 @@ enum {
     BV_OPT_L2_CHUNK_MB = 3,  /* input bytes per chunk: the chunk and its H,S,V scratch stay in L2 across the passes */
     BV_OPT_NO_HUE_TABLE = 4, /* 1: always do the HSV round trip arithmetically (testing) */
     BV_OPT_CONTOUR_POOL_CHUNKS = 5, /* chunks of the contour walk's vertex pool per frame (testing the second-walk fallback) */
-    BV_OPT_FAST_TABLES = 6, /* 1: passes 2 and 3 with per-lane replicated (bank-conflict-free) shared-memory tables; measured slower in a real step, see DESIGN.md */
-    BV_OPT_MORPH_VARIANT = 7, /* binary morphology chain: 0 register-rolling warps (default), 1 shared-memory tile filled with plain loads,
-                                 2 shared-memory tile filled by one TMA bulk copy (A-B timing, profiles/r02_morph_variants.log) */
-    BV_OPT_NO_RCP_TABLES = 8, /* 1: pass 2 looks sdiv / hdiv up in shared memory instead of computing them with the reciprocal unit (A-B timing) */
-    BV_OPT_FINAL_SV_TABLES = 9, /* pass 3 of balance -> BGR2LAB: 0 byte S'/V' tables (default); 1 float32 s, v tables; 2 8-byte {s, 1-s} / {v, trunc(255 v)} tables (A-B timing, DESIGN.md 4b) */
+    /* 6, 8 and 9 are retired (alternative balance passes that lost their measurements, DESIGN.md 4b): bv_set_option refuses them */
+    BV_OPT_MORPH_VARIANT = 7, /* binary morphology chain: 0 default choice; > 0 shared-memory tile (testing) */
     BV_OPT_MORPH_WARPS = 10, /* register-rolling morphology: row strips (= warps) per SM over the whole launch; taller strips re-compute less halo */
     BV_OPT_COUNT = 11
 };

@@ -7,8 +7,8 @@ families for the whole list of steps:
   roll<R,N,K>   morph_roll_kernel: every elementary step a square (2R+1)^2 element, R = 1 or 2, N = 1, 2 or 4 steps,
                 rows of at most 128 words (K = words per lane); one warp walks down a strip of rows
   chain<T>      morph_chain_kernel: a tile of T shared-memory rows (32..256, a multiple of 32) holding the output rows plus
-                the halo of every step; "+48k" when the launch opts in to more than 48 KiB; the TMA variant stages a
-                tile by bulk copy only when the tile's byte range is 16-byte aligned
+                the halo of every step; "+48k" when the launch opts in to more than 48 KiB.  BV_OPT_MORPH_VARIANT > 0
+                forces it onto the shapes roll would take, so that its arithmetic is tested on the module shapes
   step          morph_bits_kernel, one launch per pass of every erosion / dilation, when the chain does not qualify: a
                 GRADIENT step, a horizontal extent over 31, more than 256 tile rows or more than 200 KiB
 
@@ -139,27 +139,6 @@ def expected_morph_path(steps, batch, h, w, variant=0, sm_count=SM_COUNT, warps=
         L, R, U, D = rect_extents(kw, kh, it, h, w)
         passes.append((op, bits_passes((L, R)), bits_passes((U, D))))
     return MorphPath("step", passes=tuple(passes))
-
-
-def tma_staged_tiles(path, batch, h, w, halo_up):
-    """morph_chain_kernel<true>: {(frame, tile): staged by bulk copy} for a chain path; `frame` counts from the start of
-    the bits scratch (the stage's chunks all index one scratch image, which cudaMalloc aligns)."""
-    wpr = words_per_row(w)
-    out = {}
-    for f in range(batch):
-        for t in range(path.tiles):
-            ybase = t * path.tile_rows - halo_up
-            ya, yb = max(ybase, 0), min(ybase + path.rows, h)
-            g = ((f * h + ya) * wpr) * 4
-            d = (ya - ybase) * wpr * 4
-            nbytes = (yb - ya) * wpr * 4
-            out[(f, t)] = yb > ya and (g | d | nbytes) % 16 == 0
-    return out
-
-
-def halo_up(steps):
-    el = elementary_steps(steps) or []
-    return sum(e[3] for e in el)
 
 
 def reachable_morph_paths():
@@ -344,7 +323,7 @@ def _chain_cases():
     for i, rows in enumerate(range(32, 257, 32)):
         steps = [("dilate", 3, rows // 2 + 1, 1)] if i % 2 else [("close", 5, rows // 4 + 1, 1)]
         wide = 32 * (SMEM_DEFAULT // (8 * rows) + 1) - 5
-        for variant, w in ((1, 160), (2, 173), (1 + i % 2, wide)):
+        for variant, w in ((1, 160), (1, 173), (1, wide)):
             p = "chain<%d>%s" % (rows, "+48k" if w == wide else "")
             out.append(StageCase("chain%d_v%d_w%d" % (rows, variant, w), (2, rows * 2 + 11, w), steps, p, mask="blobs",
                                  variant=variant, seed=30 + i, group="chain_tiles"))
@@ -359,7 +338,7 @@ def _chain_cases():
     out.append(StageCase("chain_no_steps_left", (2, 50, 77), [("erode", 1, 1, 1), ("dilate", 3, 3, 0)], "chain<32>", seed=43,
                          group="chain_mixed"))
     # shared memory: above 48 KiB (width > 6144 at 32 rows), the widest tile under 200 KiB, above 200 KiB -> step
-    for variant in (0, 1, 2):
+    for variant in (0, 1):
         out.append(StageCase("chain_6145_v%d" % variant, (1, 70, 6145), [("open", 5, 5, 1)], "chain<32>+48k", variant=variant,
                              mask="blobs", seed=50 + variant, group="chain_smem"))
         out.append(StageCase("chain_12800_v%d" % variant, (1, 40, 12800), [("close", 3, 3, 1)], "chain<32>+48k",
@@ -372,10 +351,10 @@ def _chain_cases():
                          group="chain_smem"))
     out.append(StageCase("step_over_256_rows", (1, 400, 64), [("dilate", 1, 131, 1)], "step", mask="points", seed=59,
                          group="chain_smem", edges=False, nontrivial=True))
-    # TMA: wpr % 4 decides per tile whether the bulk copy or the plain loads stage it
+    # the module chain (OPEN 5x5) on the tile at row widths of whole, odd and partial words, up to the 4097 px past 48 KiB
     for w in (128, 160, 161, 200, 2208, 2209, 4097):
-        out.append(StageCase("tma_w%d" % w, (3, 75, w), [("open", 5, 5, 1)], "chain<32>" + ("+48k" if 2 * 32 * words_per_row(w) * 4 > SMEM_DEFAULT else ""),
-                             variant=2, mask="blobs", seed=60 + w % 97, group="chain_tma"))
+        out.append(StageCase("tile_w%d" % w, (3, 75, w), [("open", 5, 5, 1)], "chain<32>" + ("+48k" if 2 * 32 * words_per_row(w) * 4 > SMEM_DEFAULT else ""),
+                             variant=1, mask="blobs", seed=60 + w % 97, group="chain_widths"))
     return out
 
 

@@ -646,11 +646,14 @@ def test_stage_mask_only_shapes_outside_the_hue_table_path(ctx, shape):
         assert np.array_equal(lab[i], ccl.label_and_moments(m_ref)[1])
 
 
-@pytest.mark.parametrize("option,values", [("final_sv_tables", (1, 2)), ("morph_warps", (1, 3)), ("no_rcp_tables", (1,)),
-                                           ("fast_tables", (1,)), ("morph_variant", (1, 2)), ("no_hue_table", (1,))])
+@pytest.mark.parametrize("option,values", [("morph_warps", (1, 3)), ("morph_variant", (1,)), ("no_hue_table", (1,))])
 def test_tuning_options_do_not_change_results(ctx, option, values):
-    """Every A-B knob of the library (bv_set_option / BV_* environment variables) selects another implementation of the
-    same arithmetic: outputs are identical to the default's, on the stages the knobs act on."""
+    """Every tuning or testing knob of the library (bv_set_option / BV_* environment variables) that selects another
+    implementation of the same arithmetic leaves outputs identical to the default's, on the stages the knobs act on.
+    The retired options 6, 8 and 9 are refused."""
+    from cuauv_vision_pipeline_b200._ffi import lib
+    for retired in (6, 8, 9):
+        assert lib.bv_set_option(ctx.handle, retired, 1) == lib.BV_ERR_INVALID, retired
     frames = np.stack([synth.gen_underwater(416, 672, 900 + i) for i in range(6)])
     dev = ctx.upload(frames)
     stages = [(ctx.make_stage(balance={}, cvt="bgr2lab"), ("converted",)),

@@ -507,11 +507,10 @@ def test_min_area_rect_degenerate_contours(ctx):
         assert np.allclose([*rect[0], *rect[1], rect[2]], [*ref[0], *ref[1], ref[2]], rtol=0, atol=1e-3), (ref, rect)
 
 
-@pytest.mark.parametrize("variant", [0, 1, 2])
+@pytest.mark.parametrize("variant", [0, 1])
 @pytest.mark.parametrize("shape", [(270, 480), (479, 641), (33, 31), (1242, 2208), (96, 4096), (5, 1024)])
 def test_chain_variants_agree_with_cv2(ctx, variant, shape):
-    """The three implementations of the binary chain (register-rolling warps / shared-memory tile / tile staged by TMA)
-    against cv2 for the chains the modules use: OPEN 5x5 (bins.py:23-24), OPEN+CLOSE 5x5 (red_buoy.py:31-34), 3x3."""
+    """Both implementations of the binary chain (register-rolling warps / shared-memory tile) against cv2 for the chains the modules use: OPEN 5x5 (bins.py:23-24), OPEN+CLOSE 5x5 (red_buoy.py:31-34), 3x3."""
     ctx.set_option("morph_variant", variant)
     try:
         m = synth.mask_random(shape[0], shape[1], 11, 0.6)

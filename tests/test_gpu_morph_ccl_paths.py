@@ -187,7 +187,7 @@ def test_every_variant_and_warp_count_gives_the_default_bytes(ctx, shape):
         for f in range(b):
             assert difference(default[f], mc.cv2_steps(masks[f], steps)) is None, (steps, f)
         try:
-            for variant in (0, 1, 2):
+            for variant in (0, 1):
                 for warps in (0, 1, 2, 3, 8, 64):
                     ctx.set_option("morph_variant", variant)
                     ctx.set_option("morph_warps", warps)

@@ -60,16 +60,6 @@ def test_step_cases_cover_gradient_and_identity_steps():
         assert any(c.steps == [(op, 1, 1, 1)] for c in STAGE) and any(c.steps == [(op, 5, 5, 0)] for c in STAGE)
 
 
-def test_tma_cases_stage_some_tiles_by_bulk_copy_and_some_by_loads():
-    staged = []
-    for c in STAGE:
-        p = c.predicted()
-        if c.variant == 2 and p.kind == "chain":
-            b, h, w = c.shape
-            staged += mc.tma_staged_tiles(p, b, h, w, mc.halo_up(c.steps)).values()
-    assert True in staged and False in staged
-
-
 def test_stage_cases_cover_widths_heights_batches_and_entries():
     widths = {c.shape[2] for c in STAGE}
     assert {1, 31, 32, 33, 63, 64, 65, 1025, 2048, 2049, 4096, 4097, 6145} <= widths and max(widths) > 25600

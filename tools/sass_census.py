@@ -12,7 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "cuauv_vision_pipeline_b200", "lib", "libb200vision.so")
 KEYS = ["UBLKCP", "UTMALDG", "SYNCS", "ATOMS", "ATOMG", "RED", "LDS", "STS", "LDG", "STG", "SHFL", "BAR", "IMAD", "FFMA", "LOP3",
         "PRMT", "VIMNMX3", "HMMA", "UTCHMMA", "MUFU", "I2F", "F2I"]
-WANT = ["hist_bgr_kernel", "hist_sv_kernel", "hist_sv_fast_kernel", "final_kernel", "final_fast_kernel", "mask_from_hsv_kernel",
+WANT = ["hist_bgr_kernel", "hist_sv_kernel", "final_kernel", "mask_from_hsv_kernel",
         "ivl_build_kernel", "morph_roll_kernel", "morph_chain_kernel", "letterbox_tma_kernel", "resize_kernel", "cvt_kernel",
         "ccl_merge_kernel", "ccl_final_kernel", "contour_kernel", "min_area_rect_kernel", "rgba_to_rgb_kernel"]
 

@@ -4,7 +4,7 @@
 // Reported: SM clocks per WARP-instruction of the measured kind (clock64 per block, averaged), i.e. the reciprocal
 // throughput the colour-balance passes run against.
 //   lds8      LDS.U8  from a 256-byte table               (pass 2 / pass 3 byte tables, ~2 words per bank)
-//   lds8rep   LDS.U8  from the per-lane replica           (balance_fast.cuh layout: bank = lane, conflict-free)
+//   lds8rep   LDS.U8  from a per-lane replica             (a 128-byte row per index, lane l reads word l: bank = lane, conflict-free)
 //   lds32     LDS.32  from a 256-entry int table          (sdiv / hdiv)
 //   lds16c    LDS.U16 from a 3072-entry table             (Lab cube-root table)
 //   atoms     ATOMS.POPC.INC on a per-warp 256-bin histogram, all lanes active
